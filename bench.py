@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the pseudo-label mining step (BASELINE.json metric: Mpixel/s + fraction of HBM roofline).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" = one pass of the hot path over one target batch + one source batch
 (tools/train_ssl_uem.py:209-216 + the detached part of loss_calc_uvem, balance.py:372-396):
@@ -20,6 +20,10 @@ One JSON line is printed by rank 0 (contract in the task statement):
   parity    N = 1: the GPU step against the CPU arm's outputs on the same images; N > 1: prototype bank bit-identical
             across ranks, equal to a one-GPU run over the concatenated batch, each rank's hard labels equal to its slice
   extra     N = 1: the same resident step at BASELINE configs[2] (LoveDA shape) and configs[4] (batch 32), few steps each
+
+--dump-outputs DIR writes what the last timed step of the headline run handed back (rank 0): refined soft labels, hard
+labels, entropy, UVEM weight and the prototype bank after the step, as DIR/<name>.npy.  The inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -64,7 +68,12 @@ def parse():
     ap.add_argument("--opt", action="append", default=[], help="development: name=value for uem_set_option (repeatable)")
     ap.add_argument("--force-peer", action="store_true", help="development: N = 1 with the peer exchange kernels in the loop")
     ap.add_argument("--timeline", action="store_true", help="development: print the serial per-part timeline to stderr")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32, at most 64 MiB in all)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
 
 
 # --------------------------------------------------------------------------------------------- helpers
@@ -91,6 +100,33 @@ def step_algorithmic_bytes(wl):
     feat = wl.b * wl.k * wl.h * wl.w * 4
     target = wl.pixels * (4 * wl.c + 8 + 4 * wl.c + 8 + 4 + 4)   # soft + sup -> refined + hard + entropy + weight
     return target + feat + wl.pixels * 8 + feat                   # + target features, source labels, source features
+
+
+DUMP_BYTES = 64 << 20   # --dump-outputs: the whole dump stays below this
+
+
+def dump_sample_index(numel, cap):
+    """the flat indices written for a tensor of ``numel`` elements, at most ``cap`` of them: seeded, sorted and unique, so
+    the same on every run"""
+    return torch.unique(torch.randint(numel, (cap,), generator=torch.Generator().manual_seed(0)))
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every tensor of ``arrays`` as out_dir/<name>.npy in float32 (the labels are small integers: exact).  A tensor
+    larger than its even share of DUMP_BYTES is written as a 1-D sample, its values at dump_sample_index(numel, share).
+    Returns {name: [numel, written]}."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_BYTES // (4 * len(arrays))
+    info = {}
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > cap:
+            t = t.reshape(-1)[dump_sample_index(t.numel(), cap).to(t.device)]
+        a = t.float().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        info[name] = [int(arrays[name].numel()), int(a.size)]
+    return info
 
 
 class ClockSampler:
@@ -688,6 +724,7 @@ def nccl_pipeline(args, wl, sets, capacity, miner, dev):
     state = {"pos": 0}
 
     def run(cnt, eager=False):
+        """the next `cnt` steps; returns the set index of the last one"""
         first = state["pos"]
         state["pos"] += cnt
         cur = torch.cuda.current_stream(dev)
@@ -706,6 +743,7 @@ def nccl_pipeline(args, wl, sets, capacity, miner, dev):
             else:
                 outs[j] = phase_b(j)
             ev_b[j].record(cur)
+        return (first + cnt - 1) % n
     return run, outs, graphs is not None, per_step
 
 
@@ -744,13 +782,13 @@ def time_resident(wl, dev, rank, world, args, steps, warmup, miner=None, gen_ima
     stream = pipe.main if pipe is not None else torch.cuda.current_stream(dev)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(stream)
-    run(steps)
+    last = run(steps)
     e1.record(stream)
     barrier()
     ms = e0.elapsed_time(e1) / steps
     eager_launches = (lib.uem_kernel_launches() - l0) / steps if not graphed else (nccl_launches if pipe is None else None)
-    return {"ms": ms, "graphed": graphed, "mode": mode, "pipe": pipe, "outs": outs, "sets": sets, "inp": inp, "capacity": capacity,
-            "eager_launches": eager_launches}
+    return {"ms": ms, "graphed": graphed, "mode": mode, "pipe": pipe, "outs": outs, "last": last, "sets": sets, "inp": inp,
+            "capacity": capacity, "eager_launches": eager_launches}
 
 
 def count_step_launches(pipe):
@@ -823,6 +861,15 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms = float(t.item())
     pipe = res["pipe"]
+    if args.dump_outputs:   # before anything below runs another step
+        if rank == 0:
+            refined, hard, ent, wgt = res["outs"][res["last"]]
+            bank = pipe.proto_state if pipe is not None else miner.aligner.prototypes
+            info = dump_outputs(args.dump_outputs, {"refined": refined, "hard": hard, "entropy": ent, "uvem_weight": wgt,
+                                                    "prototypes": bank})
+            print("outputs of the last of %d timed steps (input set %d) in %s, [elements, written]: %s" % (
+                args.steps, res["last"], args.dump_outputs, json.dumps(info)), file=sys.stderr)
+        barrier()   # N > 1: the other ranks' next exchange must not wait on rank 0's copy
     exchange_status = None
     if miner is not None and miner.peer is not None:
         exchange_status = miner.peer.status()

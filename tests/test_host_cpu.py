@@ -141,6 +141,31 @@ def test_synth_is_deterministic():
     assert 0.2 < frac < 0.95  # the 7x7 edge shrink marks a large share of pixels as 'ignored'
 
 
+def test_bench_dump_is_bounded_and_repeatable(tmp_path):
+    """bench.py --dump-outputs: one float32 .npy per output, an output larger than its share written as its own values at
+    sorted, unique, seeded flat indices (the same on every run), and at most DUMP_BYTES in all."""
+    import numpy as np
+    import bench
+    g = torch.Generator().manual_seed(1)
+    arrays = {"refined": torch.rand(8, 6, 512, 512, generator=g), "hard": torch.randint(-1, 6, (8, 512, 512), generator=g),
+              "prototypes": torch.randn(6, 2048, generator=g)}
+    info = bench.dump_outputs(str(tmp_path / "a"), arrays)
+    bench.dump_outputs(str(tmp_path / "b"), arrays)
+    total = 0
+    for name in arrays:
+        x, y = np.load(tmp_path / "a" / (name + ".npy")), np.load(tmp_path / "b" / (name + ".npy"))
+        assert x.dtype == np.float32 and np.array_equal(x, y), name
+        total += x.nbytes
+    assert total <= bench.DUMP_BYTES
+    assert info["refined"] == [arrays["refined"].numel(), np.load(tmp_path / "a" / "refined.npy").size]
+    assert info["refined"][1] < info["refined"][0]
+    idx = bench.dump_sample_index(arrays["refined"].numel(), bench.DUMP_BYTES // (4 * len(arrays)))
+    assert idx.numel() == info["refined"][1] and bool((idx[1:] > idx[:-1]).all())   # sorted, no repeats
+    assert np.array_equal(np.load(tmp_path / "a" / "refined.npy"), arrays["refined"].reshape(-1)[idx].numpy())
+    assert np.array_equal(np.load(tmp_path / "a" / "hard.npy"), arrays["hard"].numpy().astype(np.float32))
+    assert np.array_equal(np.load(tmp_path / "a" / "prototypes.npy"), arrays["prototypes"].numpy())
+
+
 _WORKER = r'''
 import os, sys, torch, torch.distributed as dist
 sys.path.insert(0, os.environ["UEM_ROOT"])
