@@ -105,10 +105,8 @@ UEM_API int uem_pseudo_select_f32(const float* mask, const float* cmax, int b, i
  * uem_class_stats_decode_f32: table -> cmax (b*c) and image_min (b) as plain floats (NaN if the bad flag is set),
  * for the reference's range assert (pseudo_generation.py:71). */
 UEM_API int64_t uem_class_stats_bytes(int b, int c);
-/* development switches (A/B runs, tests): "refine_form" = 0 (pixel-pair packed column walk) | 1 (class-pair packing) |
- * -1 (the library default); the two forms of the fused label_refine kernel agree bit for bit.
+/* tuning switches (an unknown name is refused with an error):
  * "{refine,region,proto}_ctas_per_sm": cap on resident CTAs per SM (0 = occupancy limit; pipelined hosts cap the region-max kernel).
- * "pdl_pearson" (default 0): the prototype-centre and Pearson kernels are launched with programmatic stream serialization.
  * L2 eviction-priority hints (results never change): "l2_stream" (default 1) = maps a step touches exactly once (feature maps,
  * full-resolution labels, the selection's outputs and its read of the refined map) are evict_first; "l2_last_use" (default 1) =
  * the refine kernel's reads of soft / ids on the fused chain are evict_first; "l2_region" = 0 | 1 (evict_first, default) | 2
@@ -368,9 +366,9 @@ UEM_API int uem_peer_free(void* ptr);
  * forward : sums[m] += sum_px coef * CrossEntropy(upsample(x_m))[px, target]   (fp64, zeroed by the caller); the loss
  *           is (sums[0] [+ sums[1]]) / (valid + 1e-7) / heads.
  * backward: g_m (b,c,h,w) = scale[0] * d sums[m] / d x_m, every element written, deterministic (a gather per low-res
- *           cell, no atomics); scale: device scalar = grad_out / (valid + 1e-7) / heads.  ws: uem_uvem_loss_backward_ws_bytes
- *           bytes of scratch -> every pixel's softmax is evaluated once (per-block partials, then a fixed-order gather per
- *           cell); NULL -> the one-warp-per-cell form without scratch (4x the exponentials). */
+ *           cell, no atomics); scale: device scalar = grad_out / (valid + 1e-7) / heads.  ws (required, not NULL):
+ *           uem_uvem_loss_backward_ws_bytes bytes of scratch for the per-block partials (every pixel's softmax is evaluated
+ *           once, then a fixed-order gather per cell). */
 UEM_API int uem_uvem_loss_forward_f32(const float* x1, const float* x2, int b, int c, int h, int w, int H, int W,
                               const int64_t* target, const float* coef, double* sums, void* stream);
 UEM_API int64_t uem_uvem_loss_backward_ws_bytes(int b, int c, int h, int w, int heads);

@@ -51,21 +51,34 @@ def test_ctypes_signatures_match_header(built_lib):
     assert lib.uem_mine_ws_bytes(8, 6, 512, 512, 32, 32, 2048, 1025) > 8 * 6 * 32 * 32 * 4
 
 
-def test_options_and_exchange_geometry_are_host_only(built_lib):
-    """uem_set_option and the exchange-region geometry are pure host code: callable without a device; unknown options and
-    out-of-range worlds are refused with an error, not ignored."""
+def test_options_and_exchange_geometry_are_host_only_removed_options_refused(built_lib):
+    """uem_set_option and the exchange-region geometry are pure host code: callable without a device; unknown options
+    (among them the removed refine_form, refine_slot_skew and pdl_pearson) and out-of-range worlds are refused with an
+    error, not ignored."""
     from uemda_b200 import _lib
     lib = _lib.load()
-    defaults = {"l2_stream": 1, "l2_last_use": 1, "l2_region": 1, "l2_keep": 0, "refine_form": -1, "refine_ctas_per_sm": 0,
-                "region_ctas_per_sm": 0, "proto_ctas_per_sm": 0, "refine_slot_skew": 0}
+    defaults = {"l2_stream": 1, "l2_last_use": 1, "l2_region": 1, "l2_keep": 0, "refine_ctas_per_sm": 0,
+                "region_ctas_per_sm": 0, "proto_ctas_per_sm": 0}
     for name, v in defaults.items():
         assert lib.uem_set_option(name.encode(), v) == 0, name
-    assert lib.uem_set_option(b"no_such_option", 1) != 0
-    assert b"no_such_option" in lib.uem_last_error()
+    for name in ("no_such_option", "refine_form", "refine_slot_skew", "pdl_pearson"):
+        assert lib.uem_set_option(name.encode(), 1) != 0, name
+        assert name.encode() in lib.uem_last_error()
     one = lib.uem_xchg_region_bytes(1, 3, 6, 2048)
     eight = lib.uem_xchg_region_bytes(8, 3, 6, 2048)
     assert one > 3 * 6 * 2048 * 8 and (eight - 2048) == 8 * (one - 2048)   # header + depth x world x slot
     assert lib.uem_xchg_region_bytes(17, 3, 6, 2048) < 0 and lib.uem_xchg_region_bytes(2, 5, 6, 2048) < 0
+
+
+def test_uvem_loss_backward_requires_workspace(built_lib):
+    """uem_uvem_loss_backward_f32 has one form, which needs its scratch: ws = NULL is refused with an error before any
+    pointer is touched (so this runs without a device)."""
+    import ctypes
+    from uemda_b200 import _lib
+    lib = _lib.load()
+    p = ctypes.c_void_p(256)   # never dereferenced
+    assert lib.uem_uvem_loss_backward_f32(p, None, 2, 6, 8, 8, 64, 64, p, p, p, p, None, None, None) != 0
+    assert b"ws" in lib.uem_last_error()
 
 
 def test_sass_is_sm100a(built_lib):

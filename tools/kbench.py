@@ -25,13 +25,11 @@ def main():
     ap.add_argument("--iters", type=int, default=60)
     ap.add_argument("--only", default="")
     ap.add_argument("--opt", action="append", default=[], help="name=value for uem_set_option (repeatable)")
-    ap.add_argument("--refine-form", type=int, default=-1, help="0 = pixel-pair packed column walk, 1 = first form, -1 = library default")
     args = ap.parse_args()
     wl = WORKLOADS[args.workload]
     dev = torch.device("cuda", 0)
     torch.cuda.set_device(dev)
     _lib.load()
-    _lib.check(_lib.load().uem_set_option(b"refine_form", args.refine_form))
     for kv in args.opt:
         name, val = kv.split("=")
         _lib.check(_lib.load().uem_set_option(name.encode(), int(val)))

@@ -54,29 +54,28 @@ def main():
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1) / args.iters
         print("%-32s %8.3f ms/step  %8.1f Mpixel/s" % (name, ms, wl.pixels / ms / 1e3), flush=True)
-    # kernel level: the two forms of the backward (graph of 12 launches, CUDA events)
+    # kernel level: the backward alone (graph of 12 launches, CUDA events)
     from uemda_b200 import ops
     coef = torch.rand(wl.pixels, device=dev)
     scale = torch.ones(1, device=dev)
-    for name, per_cell in (("backward, per-block + gather (default)", False), ("backward, one warp per cell (round 1)", True)):
-        f = lambda s: ops.uvem_loss_backward(s["x1"].detach(), s["x2"].detach(), s["label"], coef, scale, per_cell=per_cell)  # noqa: E731
-        for s in sets:
-            f(s)
-        torch.cuda.synchronize()
-        g = torch.cuda.CUDAGraph()
-        keep = []
-        with torch.cuda.graph(g):
-            for i in range(12):
-                keep.append(f(sets[i % 3]))
+    f = lambda s: ops.uvem_loss_backward(s["x1"].detach(), s["x2"].detach(), s["label"], coef, scale)  # noqa: E731
+    for s in sets:
+        f(s)
+    torch.cuda.synchronize()
+    g = torch.cuda.CUDAGraph()
+    keep = []
+    with torch.cuda.graph(g):
+        for i in range(12):
+            keep.append(f(sets[i % 3]))
+    g.replay()
+    torch.cuda.synchronize()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    for _ in range(5):
         g.replay()
-        torch.cuda.synchronize()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        for _ in range(5):
-            g.replay()
-        e1.record()
-        torch.cuda.synchronize()
-        print("%-44s %8.1f us" % (name, e0.elapsed_time(e1) * 1e3 / 60), flush=True)
+    e1.record()
+    torch.cuda.synchronize()
+    print("%-44s %8.1f us" % ("backward, per-block + gather", e0.elapsed_time(e1) * 1e3 / 60), flush=True)
 
 
 if __name__ == "__main__":

@@ -20,7 +20,6 @@ def main():
     wl = WORKLOADS[sys.argv[1] if len(sys.argv) > 1 else "cfg2_isprs_8x6x512"]
     dev = torch.device("cuda", 0)
     lib = _lib.load()
-    lib.uem_set_option(b"refine_form", 1)
     config.strict_asserts = False
     inp = make_inputs(wl, seed=2333)
     sets = [{k: torch.roll(inp[k], i, 0).to(dev) for k in ("soft", "sup", "feat", "pred1", "pred2")} for i in range(3)]

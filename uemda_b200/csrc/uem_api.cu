@@ -6,7 +6,6 @@ static thread_local char g_err[512] = "";
 int g_uem_refine_ctas_per_sm = 0;
 int g_uem_region_ctas_per_sm = 0;
 int g_uem_proto_ctas_per_sm = 0;
-int g_uem_pdl_pearson = 0;
 int g_uem_l2_stream = 1;
 int g_uem_l2_keep = 0;
 int g_uem_l2_region = 1;

@@ -23,7 +23,6 @@ extern int g_uem_l2_region;            // hint of the region-max kernel's reads 
                                        // (default 1: the refine kernel is not faster on L2-hot inputs, the selection is, so the
                                        // refined map is the one thing worth the capacity; profiles/r02_l2_hints.txt)
 extern int g_uem_l2_last_use;          // 1: the refine kernel's reads of soft / ids (their last use in the chain) are evict_first
-extern int g_uem_pdl_pearson;          // 1: the centre and Pearson kernels are launched with programmatic stream serialization
 extern int g_uem_proto_ctas_per_sm;    // same for the prototype-sum kernel (so that a Pearson CTA fits beside it)
 void uem_note_launches(int n);  // bookkeeping for uem_kernel_launches()
 void uem_take_profile_events(void** start, void** stop);

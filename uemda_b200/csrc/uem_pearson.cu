@@ -29,10 +29,6 @@ __global__ void __launch_bounds__(256) proto_center_kernel(const float* __restri
                                                            float* __restrict__ pc, float* __restrict__ stats,
                                                            int* __restrict__ zero_ints, int n_zero) {
     const int j = blockIdx.x;
-    // programmatic dependent launch (option "pdl_pearson"): resident before the kernel that wrote the prototypes ends; the
-    // Pearson kernel behind this one may set up its barriers and tensor map while this one runs
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     if (j == 0)  // arrival counters of the k-split fold (uninitialised caller workspace)
         for (int i = threadIdx.x; i < n_zero; i += 256) zero_ints[i] = 0;
     const float* p = protos + (int64_t)j * k;
@@ -245,9 +241,6 @@ __global__ void __launch_bounds__(kTmaThreads) pearson_tma_kernel(const __grid_c
         mbar_fence_init();
         tma_prefetch_desc(&tmap);
     }
-    // programmatic dependent launch: everything above touches this CTA's shared memory and the kernel parameters only; the
-    // centred prototypes, their statistics and the zeroed arrival counters come from the preceding (centre) kernel
-    asm volatile("griddepcontrol.wait;" ::: "memory");
     __syncthreads();
 
     if (warp == kConsumers / 32) {
@@ -455,18 +448,7 @@ extern "C" int uem_pearson_dist_nchw_f32(const float* feat, int b, int k, int64_
     const bool vec = (hw % 4 == 0) && uem_aligned16(feat);
     const bool tma = vec && hw < (1 << 30) && k >= kKT;
     UEM_DISPATCH_C(m, {
-        cudaLaunchAttribute pdl_attr[1];
-        pdl_attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        pdl_attr[0].val.programmaticStreamSerializationAllowed = 1;
-        {
-            cudaLaunchConfig_t cfg = {};
-            cfg.gridDim = dim3(C, 1, 1);
-            cfg.blockDim = dim3(256, 1, 1);
-            cfg.stream = st;
-            cfg.attrs = pdl_attr;
-            cfg.numAttrs = g_uem_pdl_pearson ? 1 : 0;
-            UEM_CUDA(cudaLaunchKernelEx(&cfg, proto_center_kernel, protos, k, 1, pc, stats, arrivals, tma ? (int)(b * ptiles64) : 0));
-        }
+        proto_center_kernel<<<C, 256, 0, st>>>(protos, k, 1, pc, stats, arrivals, tma ? (int)(b * ptiles64) : 0);
         if (tma) {
             CUtensorMap tmap;
             UEM_REQUIRE(uem_make_tmap_3d_f32(&tmap, feat, (uint64_t)hw, (uint64_t)k, (uint64_t)b, (uint64_t)hw, (uint64_t)k * hw, kPT,
@@ -477,15 +459,8 @@ extern "C" int uem_pearson_dist_nchw_f32(const float* feat, int b, int k, int64_
             const int kper = ((k + KS - 1) / KS + kKT - 1) / kKT * kKT;
             const size_t smem = (size_t)kStages * (kKT * kPT + kKT * kPcStride) * 4 + 2 * kStages * 8 + (size_t)kPT * (2 + C) * 4;
             UEM_CUDA(cudaFuncSetAttribute(pearson_tma_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            cudaLaunchConfig_t cfg = {};
-            cfg.gridDim = dim3(ptiles * KS, b, 1);
-            cfg.blockDim = dim3(kTmaThreads, 1, 1);
-            cfg.dynamicSmemBytes = smem;
-            cfg.stream = st;
-            cfg.attrs = pdl_attr;
-            cfg.numAttrs = g_uem_pdl_pearson ? 1 : 0;
-            UEM_CUDA(cudaLaunchKernelEx(&cfg, pearson_tma_kernel<C>, tmap, (const float*)feat, k, (int)hw, kper, KS, (const float*)pc,
-                                        (const float*)stats, eps, reciprocal, gpart, arrivals, out, g_uem_l2_stream ? 1 : 0));
+            pearson_tma_kernel<C><<<dim3(ptiles * KS, b), kTmaThreads, smem, st>>>(tmap, feat, k, (int)hw, kper, KS, pc, stats, eps, reciprocal,
+                                                                                   gpart, arrivals, out, g_uem_l2_stream ? 1 : 0);
         } else if (vec) {
             dim3 grid(uem_div_up(hw, kPxLanes * 4), b);
             pearson_nchw_kernel<C, 4><<<grid, kPearsonThreads, 0, st>>>(feat, k, hw, pc, stats, eps, reciprocal, out);

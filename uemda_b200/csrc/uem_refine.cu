@@ -8,7 +8,7 @@
 // Compulsory traffic per pixel: read soft (4c) + sup (8), write refined (4c); everything else (three
 // low-res maps, the per-region weight table) is L2/L1 resident.
 //
-// Two kernels:
+// Two kernels, chosen from the configuration by launch_refine:
 //   * refine_col_kernel -- the default configuration (all three views, two heads, W % 4 == 0): a lane owns one or two
 //     image COLUMNS and walks down a range of rows, so the horizontal half of the bilinear interpolation is hoisted out
 //     of the row loop (one packed FFMA per class pair and row); rows arrive by per-warp cp.async three rows ahead; no
@@ -23,7 +23,6 @@
 // (pseudo_generation.py:76) fall out as a (b, c+2) stats table raised with atomicMax.
 #include "uem_common.cuh"
 #include "uem_tma.cuh"
-#include <stdlib.h>
 #include <string.h>
 
 int uem_region_table_f32(const float* src, int64_t sb, int64_t sn, int64_t sc, const int64_t* index, int b, int64_t N,
@@ -42,9 +41,6 @@ int uem_select_entropy_stats_impl(const float* mask, const uint32_t* class_stats
 #define UEM_FMUL2(a, b) __fmul2_rn(a, b)
 #define UEM_FADD2(a, b) __fadd2_rn(a, b)
 
-#ifndef UEM_ABL
-#define UEM_ABL 0   // development: ablation bits of refine_col_kernel (1 no stores, 2 no arithmetic, 4 no gather, 8 one setup, 16 no row loads)
-#endif
 namespace {
 
 constexpr int kRefineThreads = 128;
@@ -80,42 +76,11 @@ struct RefineParams {
     const float* soft;
     float* out;
     unsigned* stats;        // (b, C+2) ordered-u32: per-class max of `out`, -(min of out), bad flag; atomically raised
-    // work split of the persistent column-walk kernels: the grid is n_sm x per_sm CTAs and CTA i is the (i / n_sm)-th CTA
-    // to land on its SM.  The warp scheduler favours the older CTA's warps, so the co-resident CTAs of one SM advance at
-    // different speeds (profiles/r02_refine_cta_timeline_cfg5_by_slot.txt: 88 / 92.5 / 97 us for equal shares, the first
-    // one then leaves its SM a third empty): every CTA gets a share of the rows proportional to slot_w[its slot].
     int l2_in, l2_out;      // L2 eviction-priority hints (l2_policy kinds) of the soft / id reads and of the stores of `out`
-    int n_sm;
-    float slot_cum[5];      // cumulative, normalised: slot s owns the fraction [slot_cum[s], slot_cum[s+1]) of all rows
 };
 
-// first unit of CTA `bid` (of `grid`) under the per-slot shares; == total * bid / grid for equal shares
-__device__ __forceinline__ int64_t refine_range_begin(const RefineParams& p, int64_t total, int bid, int grid) {
-    if (p.n_sm <= 0 || grid % p.n_sm != 0 || grid / p.n_sm > 4) return total * bid / grid;
-    if (bid >= grid) return total;
-    const int slot = bid / p.n_sm, j = bid - slot * p.n_sm;
-    const double f = (double)p.slot_cum[slot] + ((double)p.slot_cum[slot + 1] - (double)p.slot_cum[slot]) * ((double)j / (double)p.n_sm);
-    int64_t u = (int64_t)(f * (double)total);
-    return u < 0 ? 0 : (u > total ? total : u);
-}
-
-// packed variant over PC class pairs
-template <int PC> __device__ __forceinline__ float exp_shifted2(float2 (&z)[PC]) {
-    float mx = fmaxf(z[0].x, z[0].y);
-#pragma unroll
-    for (int j = 1; j < PC; ++j) mx = fmaxf(mx, fmaxf(z[j].x, z[j].y));
-    const float2 nmx = make_float2(-mx, -mx), l2e = make_float2(1.4426950408889634f, 1.4426950408889634f);
-    float2 acc = make_float2(0.f, 0.f);
-#pragma unroll
-    for (int j = 0; j < PC; ++j) {
-        const float2 d = __fmul2_rn(__fadd2_rn(z[j], nmx), l2e);
-        z[j] = make_float2(ex2_approx(d.x), ex2_approx(d.y));
-        acc = __fadd2_rn(acc, z[j]);
-    }
-    return acc.x + acc.y;
-}
-
-// same, inputs already in the log2 domain (taps pre-scaled by log2 e): e_c = 2^(z_c - max z)
+// softmax numerators over PC class pairs, inputs in the log2 domain (taps pre-scaled by log2 e): e_c = 2^(z_c - max z);
+// returns their sum
 template <int PC> __device__ __forceinline__ float exp2_shifted2(float2 (&z)[PC]) {
     float mx = fmaxf(z[0].x, z[0].y);
 #pragma unroll
@@ -443,7 +408,7 @@ refine_col_kernel(const RefineParams p, const int ncols_max) {
 
     // flattened (image, strip, row) space, row fastest; this CTA owns [U0, U1)
     const int64_t total = (int64_t)p.b * nstrips * H;
-    const int64_t U0 = refine_range_begin(p, total, blockIdx.x, gridDim.x), U1 = refine_range_begin(p, total, blockIdx.x + 1, gridDim.x);
+    const int64_t U0 = total * blockIdx.x / gridDim.x, U1 = total * (blockIdx.x + 1) / gridDim.x;
     const int n = (int)(U1 - U0);
     if (n <= 0) return;
     const int bs0 = (int)(U0 / H), y0 = (int)(U0 - (int64_t)bs0 * H);
@@ -465,9 +430,6 @@ refine_col_kernel(const RefineParams p, const int ncols_max) {
 #pragma unroll
     for (int q = 0; q < NCP; ++q) { csrc[q] = nullptr; cstride[q] = 0; cvalid[q] = false; }
     auto prefetch = [&](int stage) {
-#if (UEM_ABL & 16)
-        if (stage >= 0) { if (++iy == H) { iy = 0; ++ibs; } return; }   // ablation: rows are whatever the stages hold
-#endif
         if (ibs != ibs_cur) {
             const int bi = ibs / nstrips, s = ibs - bi * nstrips;
             const int xw = s * NT * VX + wid * WC;
@@ -580,11 +542,7 @@ refine_col_kernel(const RefineParams p, const int ncols_max) {
             cur_i0 = -1;
         }
         const Lerp ly = make_lerp(y, h, p.sy);
-#if (UEM_ABL & 8)
-        if (ly.i0 != cur_i0 && it == 0) {   // ablation: only the first setup of a CTA
-#else
         if (ly.i0 != cur_i0) {
-#endif
             // new low-res row pair.  The warp's WC columns span `ncols` low-res columns: their 2 x ncols x 3C values are
             // fetched once per warp (lane -> (map, class)), pre-scaled by log2 e [/temp], and every lane then reads the
             // four corners of each of its columns as 128-bit shared-memory loads and interpolates horizontally, once.
@@ -664,11 +622,7 @@ refine_col_kernel(const RefineParams p, const int ncols_max) {
                 const uint32_t r = in_region ? lo : Ru;
                 const float4* wp = swb + r * (uint32_t)(CP / 4);
 #pragma unroll
-#if (UEM_ABL & 4)
-                for (int q = 0; q < CP / 4; ++q) swv[v][q] = make_float4(1.f, 1.f, 1.f, __uint_as_float(0x3f800000u + (r & 1u)));
-#else
                 for (int q = 0; q < CP / 4; ++q) swv[v][q] = ldg_f4_l1(wp + q);
-#endif
             }
             float sv[C][VX];
 #pragma unroll
@@ -682,18 +636,6 @@ refine_col_kernel(const RefineParams p, const int ncols_max) {
             float o[C][VX];
 #pragma unroll
             for (int v = 0; v < VX; ++v) {
-#if (UEM_ABL & 2)
-                {   // ablation: no arithmetic (loads, gather, stores and statistics stay)
-#pragma unroll
-                    for (int ci = 0; ci < C; ++ci) {
-                        const float ov = sv[ci][v] * swv[v][ci / 4].x + t2.x * A[v][ci % 3][0].x;
-                        o[ci][v] = ov;
-                        cmax[ci] = fmaxf(cmax[ci], ov);
-                        cmin = fminf(cmin, ov);
-                    }
-                    continue;
-                }
-#endif
                 float2 wgt2[PC];
                 {   // prototype view: softmax(T=1) of the up-sampled 1/distance, / (max + 1e-7) == e_c * (1 - 1e-7 S)
                     float2 z[PC];
@@ -758,9 +700,6 @@ refine_col_kernel(const RefineParams p, const int ncols_max) {
 #pragma unroll
             for (int ci = 0; ci < C; ++ci) {
                 float* dst = const_cast<float*>(ob + (int64_t)ci * HW) + idx;
-#if (UEM_ABL & 1)
-                if (o[ci][0] != 12345.678f) continue;   // ablation: no stores (the values stay live through the statistics)
-#endif
                 if constexpr (VX == 2)
                     asm volatile("st.global.L2::cache_hint.v2.f32 [%0], {%1,%2}, %3;" ::"l"(dst), "f"(o[ci][0]), "f"(o[ci][1]), "l"(pol_out) : "memory");
                 else *dst = o[ci][0];
@@ -774,421 +713,6 @@ refine_col_kernel(const RefineParams p, const int ncols_max) {
     UEM_T(5);
     if (p.stats) flush(cur_b);
     UEM_T(6);
-}
-
-// ------------------------------------------------------------------------------------------------
-// Column-walk kernel, second form (round 2; the default): same decomposition as refine_col_kernel with two columns per
-// lane, but every per-pixel quantity is a float2 over the lane's TWO PIXELS (not over a pair of classes):
-//   * the packed fp32x2 instructions (FFMA2 / FMUL2 / FADD2) then cover both pixels for every class, any class count
-//     (no padded class slot for odd C), including the final normalisation, the sums over classes and the NaN probe;
-//   * shared-memory reads of the soft planes (LDS.64) and the global stores (STG.64) are already in that layout: no
-//     re-packing moves between the class-pair and the pixel-pair form;
-//   * maxima over classes and the running class statistics use the 3-input FMNMX3 (max of C values in C/2 instructions,
-//     cmax/cmin of both pixels in one instruction per class);
-//   * the second half of the column state (D = B - A, 3C float2 per lane) lives in shared memory (DSM = 1): 128 registers
-//     -> 4 CTAs (16 warps) per SM instead of 3; it comes back as 3C conflict-free LDS.64 per row.
-// ~135 instructions per pixel in the row loop instead of ~192.  Every rounded operation is kept in the order of
-// refine_col_kernel (the class sums still add even and odd classes separately, the final sum is the same pairwise tree),
-// so the two kernels agree bit for bit (tests/test_gpu_parity.py::test_refine_kernel_forms_agree).
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ float fmax3(float a, float b, float c) {
-    float r;
-    asm("max.f32 %0, %1, %2, %3;" : "=f"(r) : "f"(a), "f"(b), "f"(c));
-    return r;
-}
-__device__ __forceinline__ float fmin3(float a, float b, float c) {
-    float r;
-    asm("min.f32 %0, %1, %2, %3;" : "=f"(r) : "f"(a), "f"(b), "f"(c));
-    return r;
-}
-// per-pixel max over C class values held as (pixel 0, pixel 1) pairs
-template <int C> __device__ __forceinline__ float2 max_over_classes(const float2 (&z)[C]) {
-    float mx = z[0].x, my = z[0].y;
-    int i = 1;
-#pragma unroll
-    for (; i + 1 < C; i += 2) { mx = fmax3(mx, z[i].x, z[i + 1].x); my = fmax3(my, z[i].y, z[i + 1].y); }
-    if (i < C) { mx = fmaxf(mx, z[i].x); my = fmaxf(my, z[i].y); }
-    return make_float2(mx, my);
-}
-// e_c = 2^(z_c - max z) for both pixels; returns S = sum e_c added as (even classes) + (odd classes), the order of
-// exp2_shifted2 over class pairs
-template <int C> __device__ __forceinline__ float2 exp2_shifted_px(float2 (&z)[C]) {
-    const float2 mx = max_over_classes<C>(z);
-    const float2 nmx = make_float2(-mx.x, -mx.y);
-    float2 ev = make_float2(0.f, 0.f), od = make_float2(0.f, 0.f);
-#pragma unroll
-    for (int c = 0; c < C; ++c) {
-        const float2 d = UEM_FADD2(z[c], nmx);
-        z[c] = make_float2(ex2_approx(d.x), ex2_approx(d.y));
-        if (c & 1) od = (c == 1) ? z[c] : UEM_FADD2(od, z[c]);
-        else ev = (c == 0) ? z[c] : UEM_FADD2(ev, z[c]);
-    }
-    return C > 1 ? UEM_FADD2(ev, od) : ev;
-}
-
-template <int C, int NT, int NS, int DSM, int MINB>
-__global__ void __launch_bounds__(NT, (MINB * 128) / NT)
-refine_col2_kernel(const RefineParams p, const int ncols_max) {
-    constexpr int CP = Lay<C>::CP, NW = NT / 32, WC = 64;
-    constexpr int TS = 3 * CP;                                   // floats per (row, low-res column) of the warp's tap scratch
-    constexpr uint32_t kPlane = (uint32_t)WC * 4u;               // bytes of one soft plane of a warp row
-    constexpr uint32_t kWarpStage = (uint32_t)WC * (4u * C + 8u);   // bytes of one row of a warp's WC columns
-    constexpr int CPP = WC / 4;                                  // 16-byte chunks per soft plane
-    constexpr int NCHUNK = CPP * C + WC / 2;                     // + the ids (2 per chunk)
-    constexpr int NCP = (NCHUNK + 31) / 32;                      // cp.async per lane and row
-    constexpr uint32_t kWarpD = DSM ? (uint32_t)(3 * C) * 32u * 8u : 0u;   // bytes of a warp's D state
-    extern __shared__ __align__(128) unsigned char smem_col[];
-    const int W = p.W, H = p.H, w = p.w, h = p.h;
-    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    const int64_t HW = (int64_t)H * W;
-    const int hw_low = h * w;
-    const int nstrips = (W + NT * 2 - 1) / (NT * 2);
-    // shared memory: [warp][stage][C planes x WC floats | WC ids]  [warp][3C][32 lanes] float2 D state  [warp][2][ncols_max][TS] taps
-    unsigned char* const wstage = smem_col + (size_t)wid * NS * kWarpStage;
-    const uint32_t dstate = smem_u32(smem_col + (size_t)NW * NS * kWarpStage + (size_t)wid * kWarpD) + (uint32_t)lane * 8u;
-    // two tap buffers per warp: the taps of the NEXT low-res row pair are prefetched (cp.async) while this one is in use
-    float* const taps_base = reinterpret_cast<float*>(smem_col + (size_t)NW * NS * kWarpStage + (size_t)NW * kWarpD) + (size_t)wid * 4 * ncols_max * TS;
-    const int tap_buf_floats = 2 * ncols_max * TS;
-
-    const int64_t total = (int64_t)p.b * nstrips * H;
-    const int64_t U0 = refine_range_begin(p, total, blockIdx.x, gridDim.x), U1 = refine_range_begin(p, total, blockIdx.x + 1, gridDim.x);
-    const int n = (int)(U1 - U0);
-    if (n <= 0) return;
-    const int bs0 = (int)(U0 / H), y0 = (int)(U0 - (int64_t)bs0 * H);
-
-    // ---- prefetch side (as in refine_col_kernel): lane l copies 16-byte chunks l, l+32, ... of a warp row
-    constexpr bool HINT = (C <= 6);
-    const uint64_t pol_in = HINT ? l2_policy(p.l2_in) : 0ull;   // last reader of soft / ids on the fused chain: evict_first
-    const uint64_t pol_out = HINT ? l2_policy(p.l2_out) : 0ull;
-    const uint32_t wstage_u32 = smem_u32(wstage) + (uint32_t)lane * 16u;
-    const uint32_t rd_base = smem_u32(wstage) + (uint32_t)lane * 8u;
-    int ibs = bs0, iy = y0, ibs_cur = -1;
-    const char* csrc[NCP];
-    uint32_t cstride[NCP];
-    bool cvalid[NCP];
-#pragma unroll
-    for (int q = 0; q < NCP; ++q) { csrc[q] = nullptr; cstride[q] = 0; cvalid[q] = false; }
-    auto prefetch = [&](int stage) {
-        if (ibs != ibs_cur) {
-            const int bi = ibs / nstrips, s = ibs - bi * nstrips;
-            const int xw = s * NT * 2 + wid * WC;
-#pragma unroll
-            for (int q = 0; q < NCP; ++q) {
-                const int k = lane + 32 * q;
-                if (k < CPP * C) {
-                    const int ci = k / CPP, x = xw + (k - ci * CPP) * 4;
-                    cvalid[q] = x < W;
-                    csrc[q] = reinterpret_cast<const char*>(p.soft + ((int64_t)bi * C + ci) * HW + (int64_t)iy * W + (cvalid[q] ? x : 0));
-                    cstride[q] = (uint32_t)W * 4u;
-                } else {
-                    const int x = xw + (k - CPP * C) * 2;
-                    cvalid[q] = (k < NCHUNK) && x < W;
-                    csrc[q] = reinterpret_cast<const char*>(p.sup + (int64_t)bi * HW + (int64_t)iy * W + (cvalid[q] ? x : 0));
-                    cstride[q] = (uint32_t)W * 8u;
-                }
-            }
-            ibs_cur = ibs;
-        }
-        const uint32_t d = wstage_u32 + (uint32_t)stage * kWarpStage;
-#pragma unroll
-        for (int q = 0; q < NCP; ++q) {
-            if constexpr (HINT) {
-                if (cvalid[q]) asm volatile("cp.async.cg.shared.global.L2::cache_hint [%0], [%1], 16, %2;" ::"r"(d + 512u * q), "l"(csrc[q]), "l"(pol_in) : "memory");
-            } else {
-                if (cvalid[q]) asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d + 512u * q), "l"(csrc[q]) : "memory");
-            }
-            csrc[q] += cstride[q];
-        }
-        if (++iy == H) { iy = 0; ++ibs; }
-    };
-#pragma unroll
-    for (int s = 0; s < NS - 1; ++s) {   // inputs only: safe before the dependency wait
-        if (s < n) prefetch(s);
-        cp_async_commit_group();
-    }
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-    const int64_t ignored_id = *p.ignored_id;
-    const uint32_t ign_lo = ((uint64_t)ignored_id >> 32) == 0 ? (uint32_t)ignored_id : 0xffffffffu;
-    const uint32_t Ru = (uint32_t)p.R;
-
-    // column state: A = pre-scaled lerp_x of low-res row i0, D = (row i1) - (row i0), as (pixel 0, pixel 1) pairs
-    float2 A[3][C];
-    float2 Dr[DSM ? 1 : 3][DSM ? 1 : C];
-    int cur_bs = -1, cur_i0 = -1, cur_b = -1;
-    int a0[2] = {0, 0}, a1[2] = {0, 0}, abase = 0, ncols = 1;
-    float l0x[2] = {0.f, 0.f}, l1x[2] = {0.f, 0.f};
-    bool active = false;
-    const float* ob = nullptr;
-    uint32_t x = 0;
-
-    float cmax[C];
-#pragma unroll
-    for (int ci = 0; ci < C; ++ci) cmax[ci] = -INFINITY;
-    float cmin = INFINITY;
-    float2 nanacc = make_float2(0.f, 0.f);
-
-    auto flush = [&](int bi) {
-        float mn = warp_min(cmin);
-        const int anybad = __any_sync(0xffffffffu, (nanacc.x != nanacc.x) | (nanacc.y != nanacc.y));
-        float mine = 0.f;
-#pragma unroll
-        for (int ci = 0; ci < C; ++ci) {
-            const float v = warp_max(cmax[ci]);
-            if (lane == ci) mine = v;
-            cmax[ci] = -INFINITY;
-        }
-        unsigned* srow = p.stats + (int64_t)bi * (C + 2);
-        if (lane < C) { if (mine > -INFINITY) atomicMax(srow + lane, f32_to_ordered(mine)); }
-        else if (lane == C) { if (mn < INFINITY) atomicMax(srow + C, f32_to_ordered(-mn)); }
-        else if (lane == C + 1) { if (anybad) atomicOr(srow + C + 1, 1u); }
-        cmin = INFINITY;
-        nanacc = make_float2(0.f, 0.f);
-    };
-
-    // region-weight gather, software-pipelined one row ahead: the ids of row it+1 are read as soon as that row has landed
-    // and its 2 x CP/4 table loads are issued before the arithmetic of row it, so their L2 latency (the table is only
-    // partly L1-resident: 35% hit rate measured) is covered by a whole row of work instead of stalling the multiply
-    float swn[2][C];
-    const float4* swb_n = nullptr;
-    auto gather = [&](int st_, bool act, const float4* tb) {
-        if (!act) return;
-        const uint32_t rd = rd_base + (uint32_t)st_ * kWarpStage;
-        int64_t rid[2];
-        asm volatile("ld.shared.v2.b64 {%0,%1}, [%2];" : "=l"(rid[0]), "=l"(rid[1]) : "r"(rd + (uint32_t)lane * 8u + (uint32_t)C * kPlane));
-#pragma unroll
-        for (int v = 0; v < 2; ++v) {
-            // multiplicative outside the ignored id; the ignored id and any id outside [0,R) go to the all-ones sentinel row R
-            const uint32_t lo = (uint32_t)rid[v], hi = (uint32_t)((uint64_t)rid[v] >> 32);
-            const bool in_region = (hi == 0u) & (lo < Ru) & (lo != ign_lo);
-            const uint32_t r = in_region ? lo : Ru;
-            const float* wp = reinterpret_cast<const float*>(tb + r * (uint32_t)(CP / 4));
-            // only the C live floats of the row: 128-bit loads, then one 64- or 32-bit load for a tail of 2 or 1
-#pragma unroll
-            for (int q = 0; q < C / 4; ++q) {
-                const float4 t = ldg_f4_l1(reinterpret_cast<const float4*>(wp) + q);
-                swn[v][4 * q] = t.x; swn[v][4 * q + 1] = t.y; swn[v][4 * q + 2] = t.z; swn[v][4 * q + 3] = t.w;
-            }
-            if constexpr (C % 4 == 3) {
-                const float4 t = ldg_f4_l1(reinterpret_cast<const float4*>(wp) + C / 4);
-                swn[v][C - 3] = t.x; swn[v][C - 2] = t.y; swn[v][C - 1] = t.z;
-            } else if constexpr (C % 4 == 2) {
-                asm volatile("ld.global.nc.L1::evict_last.v2.f32 {%0,%1}, [%2];" : "=f"(swn[v][C - 2]), "=f"(swn[v][C - 1]) : "l"(wp + (C & ~3)));
-            } else if constexpr (C % 4 == 1) {
-                asm volatile("ld.global.nc.L1::evict_last.f32 %0, [%1];" : "=f"(swn[v][C - 1]) : "l"(wp + (C & ~3)));
-            }
-        }
-    };
-    // geometry of an (image, strip) unit: is this lane inside the image, and which table does it gather from
-    auto lane_geom = [&](int bsu, bool& act, const float4*& tb) {
-        const int bi = bsu / nstrips, s = bsu - bi * nstrips;
-        act = (s * NT * 2 + wid * WC + lane * 2) < W;
-        tb = reinterpret_cast<const float4*>(p.sw + (int64_t)bi * (p.R + 1) * CP);
-    };
-
-    // ---- low-res taps.  The warp's 64 columns span `ncols` low-res columns; their 2 rows x ncols x 3C values are copied
-    // (lane -> (map, class), raw) into a tap buffer with 4-byte cp.async.  The copy for the NEXT row pair is issued right
-    // after a setup, ~H/h rows before it is needed, so its L2 / DRAM round trips (two dependent ones when issued on
-    // demand: 8% of all warp stall samples in profiles/r02_ncu_refine_col2.txt) disappear behind the row loop.
-    auto tap_fetch_async = [&](float* buf, int bsu, int i0u, int i1u) {
-        if (lane >= 3 * C) return;
-        const int bi = bsu / nstrips, su = bsu - bi * nstrips;
-        const int xw = su * NT * 2 + wid * WC;
-        const int ab = make_lerp(min(xw, W - 1), w, p.sx).i0;
-        const int nc = make_lerp(min(xw + WC - 1, W - 1), w, p.sx).i1 - ab + 1;
-        const int m = lane / C, ci = lane - m * C;
-        const float* plane = p.maps[m] + ((int64_t)bi * C + ci) * hw_low + ab;
-        const float* r0 = plane + i0u * w;
-        const float* r1 = plane + i1u * w;
-        float* dst = buf + m * CP + ci;
-        for (int j = 0; j < nc; ++j) {
-            cp_async_4(dst + j * TS, r0 + j);
-            cp_async_4(dst + (ncols_max + j) * TS, r1 + j);
-        }
-    };
-    int tap_cur = 0;                  // buffer the current column state was built from
-    int pref_bs = -1, pref_i0 = -1, pref_it = 0;   // what the other buffer holds (or will hold), and when it was issued
-
-    int bs = bs0, y = y0;
-    int stage = 0, pstage = NS - 1;
-    {   // row 0's gather
-        cp_async_wait_group<NS - 2>();
-        __syncwarp();
-        bool act0;
-        lane_geom(bs0, act0, swb_n);
-        gather(0, act0, swb_n);
-    }
-    for (int it = 0; it < n; ++it) {
-        __syncwarp();
-        if (it + NS - 1 < n) prefetch(pstage);
-        cp_async_commit_group();
-        if (bs != cur_bs) {
-            const int bi = bs / nstrips, s = bs - bi * nstrips;
-            if (bi != cur_b) {
-                if (cur_b >= 0 && p.stats) flush(cur_b);
-                cur_b = bi;
-            }
-            const int xw = s * NT * 2 + wid * WC;
-            x = (uint32_t)(xw + lane * 2);
-            active = (int)x < W;     // W is even: the lane's two columns are both inside or both outside
-#pragma unroll
-            for (int v = 0; v < 2; ++v) {
-                const Lerp lx = make_lerp(active ? (int)x + v : W - 1, w, p.sx);
-                a0[v] = lx.i0; a1[v] = lx.i1; l0x[v] = lx.l0; l1x[v] = lx.l1;
-            }
-            abase = make_lerp(min(xw, W - 1), w, p.sx).i0;
-            ncols = make_lerp(min(xw + WC - 1, W - 1), w, p.sx).i1 - abase + 1;
-            ob = p.out + (int64_t)bi * C * HW;
-            cur_bs = bs;
-            cur_i0 = -1;
-        }
-        const Lerp ly = make_lerp(y, h, p.sy);
-        if (ly.i0 != cur_i0) {
-            // new low-res row pair: the warp fetches the 2 x ncols x 3C values its 64 columns span (lane -> (map, class)),
-            // pre-scaled by log2 e [/temp]; every lane then interpolates its two columns horizontally, once
-            cur_i0 = ly.i0;
-            __syncwarp();
-            if (pref_bs == bs && pref_i0 == ly.i0) {
-                tap_cur ^= 1;                                   // prefetched after the previous setup
-                if (it - pref_it < NS) cp_async_wait_group<0>();   // issued too recently for the row loop's waits to cover it
-            } else {                                            // first setup of this CTA: fetch on demand
-                tap_fetch_async(taps_base + tap_cur * tap_buf_floats, bs, ly.i0, ly.i1);
-                cp_async_commit_group();
-                cp_async_wait_group<0>();
-            }
-            __syncwarp();
-            const float* taps = taps_base + tap_cur * tap_buf_floats;
-#pragma unroll
-            for (int m = 0; m < 3; ++m) {
-                const float sc = p.map_scale[m];   // log2 e [/temp], applied to the raw taps exactly as before the lerp
-                float ta[2][C], td[2][C];
-#pragma unroll
-                for (int v = 0; v < 2; ++v) {
-                    const float* t00 = taps + (a0[v] - abase) * TS + m * CP;
-                    const float* t01 = taps + (a1[v] - abase) * TS + m * CP;
-                    float v00[CP], v01[CP], v10[CP], v11[CP];
-                    load_tap<C>(t00, v00);
-                    load_tap<C>(t01, v01);
-                    load_tap<C>(t00 + ncols_max * TS, v10);
-                    load_tap<C>(t01 + ncols_max * TS, v11);
-#pragma unroll
-                    for (int ci = 0; ci < C; ++ci) {   // the rounded operations of refine_col_kernel, per component
-                        const float a = __fmaf_rn(l1x[v], __fmul_rn(v01[ci], sc), __fmul_rn(l0x[v], __fmul_rn(v00[ci], sc)));
-                        const float bq = __fmaf_rn(l1x[v], __fmul_rn(v11[ci], sc), __fmul_rn(l0x[v], __fmul_rn(v10[ci], sc)));
-                        ta[v][ci] = a;
-                        td[v][ci] = __fadd_rn(bq, -a);
-                    }
-                }
-#pragma unroll
-                for (int ci = 0; ci < C; ++ci) {
-                    A[m][ci] = make_float2(ta[0][ci], ta[1][ci]);
-                    if constexpr (DSM) {
-                        asm volatile("st.shared.v2.f32 [%0], {%1,%2};" ::"r"(dstate + (uint32_t)(m * C + ci) * 256u), "f"(td[0][ci]), "f"(td[1][ci]) : "memory");
-                    } else {
-                        Dr[DSM ? 0 : m][DSM ? 0 : ci] = make_float2(td[0][ci], td[1][ci]);
-                    }
-                }
-            }
-            {   // where is the next setup?  the first later row of this unit with another low-res row pair, or the next unit
-                int yn = y + 1;
-                while (yn < H && make_lerp(yn, h, p.sy).i0 == ly.i0) ++yn;
-                const int it_n = it + (yn - y);
-                pref_bs = -1;
-                if (it_n < n) {
-                    const int nbs = yn < H ? bs : bs + 1;
-                    const Lerp ln = make_lerp(yn < H ? yn : 0, h, p.sy);
-                    __syncwarp();   // every lane has read its taps of the buffer that is overwritten now (two setups ago)
-                    tap_fetch_async(taps_base + (tap_cur ^ 1) * tap_buf_floats, nbs, ln.i0, ln.i1);
-                    pref_bs = nbs; pref_i0 = ln.i0; pref_it = it;
-                }
-            }
-        }
-        cp_async_wait_group<NS - 2>();   // rows it and it+1 have landed (this lane's chunks ...
-        __syncwarp();                    // ... and the other lanes': a row is read across lanes)
-        if (active) {
-            const uint32_t rd = rd_base + (uint32_t)stage * kWarpStage;   // this lane's two floats of plane 0
-            float2 sv[C];
-#pragma unroll
-            for (int ci = 0; ci < C; ++ci)
-                asm volatile("ld.shared.v2.f32 {%0,%1}, [%2];" : "=f"(sv[ci].x), "=f"(sv[ci].y) : "r"(rd + (uint32_t)ci * kPlane));
-            const float2 t2 = make_float2(ly.l1, ly.l1);
-            auto dstate_of = [&](int m, int ci) -> float2 {
-                if constexpr (DSM) {
-                    float2 d;
-                    asm volatile("ld.shared.v2.f32 {%0,%1}, [%2];" : "=f"(d.x), "=f"(d.y) : "r"(dstate + (uint32_t)(m * C + ci) * 256u));
-                    return d;
-                } else {
-                    return Dr[DSM ? 0 : m][DSM ? 0 : ci];
-                }
-            };
-            float2 wgt[C];
-            {   // prototype view: softmax(T=1) of the up-sampled 1/distance, / (max + 1e-7) == e_c * (1 - 1e-7 S)
-                float2 z[C];
-#pragma unroll
-                for (int ci = 0; ci < C; ++ci) z[ci] = UEM_FFMA2(t2, dstate_of(0, ci), A[0][ci]);
-                const float2 S = exp2_shifted_px<C>(z);
-                const float2 rs = UEM_FFMA2(make_float2(-1e-7f, -1e-7f), S, make_float2(1.0f, 1.0f));
-#pragma unroll
-                for (int ci = 0; ci < C; ++ci) wgt[ci] = UEM_FMUL2(z[ci], rs);
-            }
-            {   // prediction view: mean of the two heads' softmax(logits/temp), / (max + 1e-7), scaled through by S1*S2
-                float2 z[C], z2[C];
-#pragma unroll
-                for (int ci = 0; ci < C; ++ci) {
-                    z[ci] = UEM_FFMA2(t2, dstate_of(1, ci), A[1][ci]);
-                    z2[ci] = UEM_FFMA2(t2, dstate_of(2, ci), A[2][ci]);
-                }
-                const float2 S1 = exp2_shifted_px<C>(z);
-                const float2 S2 = exp2_shifted_px<C>(z2);
-#pragma unroll
-                for (int ci = 0; ci < C; ++ci) z[ci] = UEM_FFMA2(z[ci], S2, UEM_FMUL2(z2[ci], S1));
-                float2 mx = max_over_classes<C>(z);
-                mx = make_float2(fmaxf(mx.x, 0.f), fmaxf(mx.y, 0.f));
-                const float2 den = UEM_FFMA2(make_float2(2e-7f, 2e-7f), UEM_FMUL2(S1, S2), mx);
-                const float2 inv = make_float2(rcp_approx(den.x), rcp_approx(den.y));
-#pragma unroll
-                for (int ci = 0; ci < C; ++ci) wgt[ci] = UEM_FFMA2(z[ci], inv, wgt[ci]);
-            }
-#pragma unroll
-            for (int ci = 0; ci < C; ++ci) wgt[ci] = UEM_FMUL2(wgt[ci], make_float2(swn[0][ci], swn[1][ci]));   // gathered one row ago
-            // soft' = w*soft / (sum + 1e-7)   (alignment.py:291-292, :324-325); pairwise tree over class pairs
-            float2 o[C];
-#pragma unroll
-            for (int ci = 0; ci < C; ++ci) o[ci] = UEM_FMUL2(wgt[ci], sv[ci]);
-            constexpr int PC = Lay<C>::PC;
-            float2 ps[PC];
-#pragma unroll
-            for (int j = 0; j < PC; ++j) ps[j] = (2 * j + 1 < C) ? UEM_FADD2(o[2 * j], o[2 * j + 1]) : o[2 * j];
-#pragma unroll
-            for (int st2 = 1; st2 < PC; st2 *= 2)
-#pragma unroll
-                for (int j = 0; j + st2 < PC; j += 2 * st2) ps[j] = UEM_FADD2(ps[j], ps[j + st2]);
-            const float2 ssum = ps[0];
-            const float2 sden = UEM_FADD2(ssum, make_float2(1e-7f, 1e-7f));
-            const float2 inv = make_float2(rcp_approx(sden.x), rcp_approx(sden.y));
-            nanacc = UEM_FFMA2(ssum, make_float2(0.f, 0.f), nanacc);   // s*0 accumulates to NaN iff a row sum was inf/NaN
-            const uint32_t idx = (uint32_t)y * (uint32_t)W + x;
-#pragma unroll
-            for (int ci = 0; ci < C; ++ci) {
-                const float2 ov = UEM_FMUL2(o[ci], inv);
-                cmax[ci] = fmax3(cmax[ci], ov.x, ov.y);
-                cmin = fmin3(cmin, ov.x, ov.y);
-                if constexpr (HINT)
-                    asm volatile("st.global.L2::cache_hint.v2.f32 [%0], {%1,%2}, %3;" ::"l"(const_cast<float*>(ob + (int64_t)ci * HW) + idx), "f"(ov.x), "f"(ov.y), "l"(pol_out) : "memory");
-                else *reinterpret_cast<float2*>(const_cast<float*>(ob + (int64_t)ci * HW) + idx) = ov;
-            }
-        }
-        if (it + 1 < n) {   // the next row's region weights: a whole row of work covers their latency
-            const int nst = (stage + 1 == NS) ? 0 : stage + 1;
-            bool actn = active;
-            if (y + 1 == H) lane_geom(bs + 1, actn, swb_n);   // the next row opens a new (image, strip)
-            gather(nst, actn, swb_n);
-        }
-        if (++y == H) { y = 0; ++bs; }
-        pstage = stage;
-        if (++stage == NS) stage = 0;
-    }
-    if (p.stats) flush(cur_b);
 }
 
 // superpixel-view weight of every (image, region): softmax(region_max/temp) / (max + 1e-7)  (alignment.py:252-253)
@@ -1273,31 +797,15 @@ static int sm_count() {
     return n;
 }
 
-// pdl: launch with programmatic stream serialization (the kernel must execute griddepcontrol.wait before it touches
-// anything the preceding kernel of the stream writes)
 template <typename K>
-static int launch_persistent(K kernel, const RefineParams& p, int threads, size_t smem, cudaStream_t st, bool pdl = false) {
+static int launch_persistent(K kernel, const RefineParams& p, int threads, size_t smem, cudaStream_t st) {
     if (smem > 48 * 1024) UEM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 0;
     UEM_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
     if (per_sm < 1) per_sm = 1;
     const int64_t total_rows = (int64_t)p.b * p.H;
     const int grid = (int)min(total_rows, (int64_t)sm_count() * per_sm);
-    if (!pdl) {
-        kernel<<<grid, threads, smem, st>>>(p);
-        return 0;
-    }
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid, 1, 1);
-    cfg.blockDim = dim3(threads, 1, 1);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    UEM_CUDA(cudaLaunchKernelEx(&cfg, kernel, p));
+    kernel<<<grid, threads, smem, st>>>(p);
     return 0;
 }
 
@@ -1311,84 +819,6 @@ static int launch_persistent(K kernel, const RefineParams& p, int threads, size_
 #ifndef UEM_REFINE_COL_VX
 #define UEM_REFINE_COL_VX 2
 #endif
-// per-slot shares of the rows (see RefineParams::slot_cum).  Measured speeds of the 1st / 2nd / 3rd CTA of an SM at equal
-// shares: 1 : 0.95 : 0.905 (config 5), 1 : 0.955 : 0.92 (config 2); "refine_slot_skew" (uem_set_option, per mille of the
-// spread between first and last slot, 100 = +-5 %) sets it; default 0 = equal shares.
-static int g_refine_slot_skew = 0;   // measured: the per-slot finish times even out, the launch does not get shorter (r02_kbench_refine_slot_skew.txt)
-static void refine_slot_shares(RefineParams& p, int grid, int per_sm) {
-    p.n_sm = 0;
-    if (per_sm < 2 || per_sm > 4 || grid != sm_count() * per_sm || g_refine_slot_skew == 0) return;
-    p.n_sm = sm_count();
-    float w[4], sum = 0.f;
-    for (int s = 0; s < per_sm; ++s) {
-        w[s] = 1.0f + 0.001f * (float)g_refine_slot_skew * (0.5f - (float)s / (float)(per_sm - 1));   // +skew/2 .. -skew/2
-        sum += w[s];
-    }
-    p.slot_cum[0] = 0.f;
-    for (int s = 0; s < per_sm; ++s) p.slot_cum[s + 1] = p.slot_cum[s] + w[s] / sum;
-    p.slot_cum[per_sm] = 1.0f;
-}
-
-#ifndef UEM_REFINE_COL2_DSM
-#define UEM_REFINE_COL2_DSM 1
-#endif
-#ifndef UEM_REFINE_COL2_MINB
-#define UEM_REFINE_COL2_MINB 3
-#endif
-#ifndef UEM_REFINE_COL2_NS
-#define UEM_REFINE_COL2_NS 5   // rows in flight per warp: the gather of row it+1 needs that row landed, 3 more stay in flight
-#endif
-// second form of the column walk (pixel-pair packing; see refine_col2_kernel).  UEM_REFINE_KERNEL=col in the environment
-// selects the first form (A/B runs and the bit-equality test of the two forms).
-template <int C>
-static int launch_refine_col2(RefineParams p, cudaStream_t st, bool pdl, bool* done) {
-    constexpr int NT = UEM_REFINE_COL_NT, NS = UEM_REFINE_COL2_NS, DSM = UEM_REFINE_COL2_DSM, MINB = UEM_REFINE_COL2_MINB;
-    *done = false;
-    constexpr float kL2E = 1.4426950408889634f;
-    p.map_scale[0] = kL2E;
-    p.map_scale[1] = p.map_scale[2] = (float)(1.4426950408889634 / (double)p.temp);
-    int ncols_max = (int)(63 * p.sx) + 3;   // low-res columns a warp's 64 image columns can span (+1 for the right neighbour)
-    if (ncols_max > p.w) ncols_max = p.w;
-    const size_t smem = (size_t)NS * NT * 2 * (4 * C + 8) + (DSM ? (size_t)NT * 3 * C * 8 : 0) +
-                        (size_t)(NT / 32) * 4 * ncols_max * 3 * cp_of(C) * 4;   // stages | D state | 2 tap buffers per warp
-    if (smem > 100 * 1024 || (int64_t)p.H * p.W >= ((int64_t)1 << 31)) return 0;   // the first form / generic kernels take it
-    auto kernel = refine_col2_kernel<C, NT, NS, DSM, MINB>;
-    if (smem > 48 * 1024) UEM_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int per_sm = 0;
-    UEM_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, NT, smem));
-    if (per_sm < 1) per_sm = 1;
-    if (g_uem_refine_ctas_per_sm > 0 && per_sm > g_uem_refine_ctas_per_sm) per_sm = g_uem_refine_ctas_per_sm;
-    const int nstrips = (p.W + NT * 2 - 1) / (NT * 2);
-    const int64_t total = (int64_t)p.b * nstrips * p.H;
-    const int grid = (int)min(total, (int64_t)sm_count() * per_sm);
-    refine_slot_shares(p, grid, per_sm);
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid, 1, 1);
-    cfg.blockDim = dim3(NT, 1, 1);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl ? 1 : 0;
-    UEM_CUDA(cudaLaunchKernelEx(&cfg, kernel, p, ncols_max));
-    *done = true;
-    return 0;
-}
-
-#ifndef UEM_REFINE_DEFAULT_FORM
-#define UEM_REFINE_DEFAULT_FORM 1   // measured on B200 (profiles/r02_kbench_refine_forms.txt): the first form is still the faster one
-#endif
-static int g_refine_form = -1;   // 0 = second form (pixel-pair packing), 1 = first form (class-pair packing)
-static bool refine_first_form() {
-    if (g_refine_form < 0) {
-        const char* e = getenv("UEM_REFINE_KERNEL");
-        g_refine_form = (e && strcmp(e, "col2") == 0) ? 0 : UEM_REFINE_DEFAULT_FORM;
-    }
-    return g_refine_form == 1;
-}
-
 template <int C>
 static int launch_refine_col(RefineParams p, cudaStream_t st, bool pdl, bool* done) {
     // two columns per lane while their state fits 168 registers (c <= 6); 7 and 8 classes would spill: one column
@@ -1411,7 +841,6 @@ static int launch_refine_col(RefineParams p, cudaStream_t st, bool pdl, bool* do
     const int nstrips = (p.W + NT * VX - 1) / (NT * VX);
     const int64_t total = (int64_t)p.b * nstrips * p.H;
     const int grid = (int)min(total, (int64_t)sm_count() * per_sm);
-    refine_slot_shares(p, grid, per_sm);
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(grid, 1, 1);
     cfg.blockDim = dim3(NT, 1, 1);
@@ -1433,7 +862,7 @@ static int launch_refine(int views, const float* simi, const float* pred1, const
                          int c, int H, int W, float temp, float* out, unsigned* stats, float* sw_ws, cudaStream_t st,
                          bool weights_ready = false, bool pdl = false) {
     // weights_ready: sw_ws already holds the per-region weights (fused tail of the region-max kernel); pdl: that kernel
-    // directly precedes this launch in the stream, so the TMA kernel may overlap its prologue with it
+    // directly precedes this launch in the stream, so the column-walk kernel may overlap its prologue with it
     UEM_REQUIRE(soft && out && b > 0 && H > 0 && W > 0, "uem_label_refine_f32: bad arguments");
     UEM_REQUIRE(views > 0 && views < 8, "uem_label_refine_f32: views must be a non-empty mask of UEM_VIEW_*");
     UEM_REQUIRE(temp > 0.f, "uem_label_refine_f32: temp must be > 0");  // alignment.py:313
@@ -1480,8 +909,7 @@ static int launch_refine(int views, const float* simi, const float* pred1, const
         uem_take_profile_events(&ev0, &ev1);
         if (ev0) UEM_CUDA(cudaEventRecord((cudaEvent_t)ev0, st));
         bool done = false;
-        if (colwalk && !refine_first_form()) rc = launch_refine_col2<C>(p, st, pdl && weights_ready && !ev0, &done);
-        if (colwalk && !done && rc == 0) rc = launch_refine_col<C>(p, st, pdl && weights_ready && !ev0, &done);
+        if (colwalk) rc = launch_refine_col<C>(p, st, pdl && weights_ready && !ev0, &done);
         if (!done && rc == 0) {
             const int vecw = vec ? 4 : 1;
             const size_t smem = (size_t)(w + 2) * Lay<C>::STRIDE * 4 + (size_t)C * kRefineThreads * vecw * 4 + (size_t)kRefineThreads * vecw * 8;
@@ -1509,15 +937,12 @@ extern "C" __attribute__((visibility("default"))) int uem_debug_refine_timing(un
 extern "C" int uem_set_option(const char* name, int value) {
     UEM_REQUIRE(name, "uem_set_option: NULL name");
     if (strcmp(name, "refine_ctas_per_sm") == 0) { g_uem_refine_ctas_per_sm = value; return 0; }
-    if (strcmp(name, "refine_slot_skew") == 0) { g_refine_slot_skew = value; return 0; }
     if (strcmp(name, "region_ctas_per_sm") == 0) { g_uem_region_ctas_per_sm = value; return 0; }
     if (strcmp(name, "proto_ctas_per_sm") == 0) { g_uem_proto_ctas_per_sm = value; return 0; }
-    if (strcmp(name, "pdl_pearson") == 0) { g_uem_pdl_pearson = value ? 1 : 0; return 0; }
     if (strcmp(name, "l2_stream") == 0) { g_uem_l2_stream = value ? 1 : 0; return 0; }
     if (strcmp(name, "l2_keep") == 0) { g_uem_l2_keep = value == 2 ? 2 : 0; return 0; }
     if (strcmp(name, "l2_region") == 0) { g_uem_l2_region = (value >= 0 && value <= 2) ? value : 0; return 0; }
     if (strcmp(name, "l2_last_use") == 0) { g_uem_l2_last_use = value ? 1 : 0; return 0; }
-    if (strcmp(name, "refine_form") == 0) { g_refine_form = value < 0 ? -1 : (value ? 1 : 0); return 0; }   // -1: back to the default
     return uem_fail("uem_set_option: unknown option '%s'", name);
 }
 

@@ -164,108 +164,15 @@ __device__ __forceinline__ int first_with_i0_ge(int i, int in_size, int out_size
     return y;   // == out_size when no such index
 }
 
-// Backward: grid = (w, h, b), one warp (32 threads) per low-res cell.
-template <int C, int NM>
-__global__ void __launch_bounds__(32) uvem_ce_grad_kernel(const float* __restrict__ x1, const float* __restrict__ x2, int h, int w, int H,
-                                                          int W, float sy, float sx, const int64_t* __restrict__ target,
-                                                          const float* __restrict__ coef, const float* __restrict__ scale,
-                                                          float* __restrict__ g1, float* __restrict__ g2) {
-    constexpr float kL2E = 1.4426950408889634f;
-    const int j = blockIdx.x, i = blockIdx.y, bi = blockIdx.z, lane = threadIdx.x;
-    const int hw_low = h * w;
-    const int64_t HW = (int64_t)H * W;
-    const float* maps[2] = {x1, x2};
-    float* grads[2] = {g1, g2};
-    // footprint: pixels whose (i0, i1) x (a0, a1) contains (i, j): i0 in {i-1, i}
-    const int ylo = first_with_i0_ge(i - 1, h, H, sy), yhi = first_with_i0_ge(i + 1, h, H, sy);   // [ylo, yhi)
-    const int xlo = first_with_i0_ge(j - 1, w, W, sx), xhi = first_with_i0_ge(j + 1, w, W, sx);
-    // the footprint splits into four quadrants around (first row with i0 >= i, first column with a0 >= j); inside a
-    // quadrant every pixel interpolates from the SAME 2x2 block of the neighbourhood, so the taps are fixed registers
-    const int ymid = first_with_i0_ge(i, h, H, sy), xmid = first_with_i0_ge(j, w, W, sx);
-    // 3x3 low-res neighbourhood of every (head, class), pre-scaled by log2 e (clamped loads: the clamped border pixel
-    // has i1 == i0 and reads the same value twice, exactly like the forward)
-    float nb[NM][C][3][3];
-#pragma unroll
-    for (int m = 0; m < NM; ++m)
-#pragma unroll
-        for (int ci = 0; ci < C; ++ci)
-#pragma unroll
-            for (int dy = 0; dy < 3; ++dy)
-#pragma unroll
-                for (int dx = 0; dx < 3; ++dx) {
-                    const int ii = min(max(i + dy - 1, 0), h - 1), jj = min(max(j + dx - 1, 0), w - 1);
-                    nb[m][ci][dy][dx] = __ldg(maps[m] + ((int64_t)bi * C + ci) * hw_low + ii * w + jj) * kL2E;
-                }
-    float acc[NM][C];
-#pragma unroll
-    for (int m = 0; m < NM; ++m)
-#pragma unroll
-        for (int ci = 0; ci < C; ++ci) acc[m][ci] = 0.f;
-
-#pragma unroll
-    for (int qy = 0; qy < 2; ++qy)
-#pragma unroll
-        for (int qx = 0; qx < 2; ++qx) {
-            const int y0 = qy ? ymid : ylo, y1 = qy ? yhi : ymid, x0 = qx ? xmid : xlo, x1 = qx ? xhi : xmid;
-            const int fw = x1 - x0, fh = y1 - y0;
-            if (fw <= 0 || fh <= 0) continue;
-            const int npx = fw * fh;
-            int fy = 0, fx = lane;
-            while (fx >= fw) { fx -= fw; ++fy; }
-            for (int q = lane; q < npx; q += 32) {
-                const int y = y0 + fy, x = x0 + fx;
-                const int64_t px = (int64_t)bi * HW + (int64_t)y * W + x;
-                const float cf = __ldg(coef + px);
-                if (cf != 0.f) {
-                    const Lerp ly = make_lerp(y, h, sy), lx = make_lerp(x, w, sx);
-                    // weight of this pixel on cell (i, j): both taps land on it at the clamped border (i0 == i1)
-                    const float wy = (ly.i0 == i ? ly.l0 : 0.f) + (ly.i1 == i ? ly.l1 : 0.f);
-                    const float wx = (lx.i0 == j ? lx.l0 : 0.f) + (lx.i1 == j ? lx.l1 : 0.f);
-                    const float wgt = wy * wx * cf;
-                    const int t = (int)__ldg(target + px);
-#pragma unroll
-                    for (int m = 0; m < NM; ++m) {
-                        float z[C];
-                        float mx = -INFINITY;
-#pragma unroll
-                        for (int ci = 0; ci < C; ++ci) {
-                            z[ci] = ly.l0 * (lx.l0 * nb[m][ci][qy][qx] + lx.l1 * nb[m][ci][qy][qx + 1]) +
-                                    ly.l1 * (lx.l0 * nb[m][ci][qy + 1][qx] + lx.l1 * nb[m][ci][qy + 1][qx + 1]);
-                            mx = fmaxf(mx, z[ci]);
-                        }
-                        float S = 0.f;
-#pragma unroll
-                        for (int ci = 0; ci < C; ++ci) { z[ci] = ex2_approx(z[ci] - mx); S += z[ci]; }
-                        float r = rcp_approx(S);
-                        r = fmaf(r, fmaf(-S, r, 1.0f), r);
-                        const float k = wgt * r;
-#pragma unroll
-                        for (int ci = 0; ci < C; ++ci) acc[m][ci] = fmaf(k, z[ci], acc[m][ci]) - ((t == ci) ? wgt : 0.f);
-                    }
-                }
-                fx += 32;
-                while (fx >= fw) { fx -= fw; ++fy; }
-            }
-        }
-    const float sc = __ldg(scale);
-#pragma unroll
-    for (int m = 0; m < NM; ++m)
-#pragma unroll
-        for (int ci = 0; ci < C; ++ci) {
-            const float v = warp_sum(acc[m][ci]);
-            if (lane == 0) grads[m][((int64_t)bi * C + ci) * hw_low + i * w + j] = v * sc;
-        }
-}
-
 // ------------------------------------------------------------------------------------------------
-// Backward, second form (round 2, the default): every pixel's softmax is evaluated ONCE.
+// Backward: every pixel's softmax is evaluated ONCE.
 // The full-resolution image splits into h x w "blocks": block (qi, qj) = the pixels whose interpolation starts at low-res
 // (qi, qj), i.e. that interpolate from the 2x2 corner cells (qi | qi+1, qj | qj+1).  Pass 1: one warp per block keeps the
 // four corners' logits in registers, walks its ~H/h x W/w pixels, and accumulates for the 4 corners x heads x classes
 // w_y * w_x * coef * (p_c - [c == target]) in per-lane registers; one warp reduction, then 4 * NM * C plain stores into a
 // per-block partial table.  Pass 2: every low-res cell adds the (at most 4 blocks x corners) partials that point at it,
-// in a fixed order.  No atomics anywhere: the gradient is bit-reproducible run to run; 4x fewer exponentials than the
-// per-cell gather above (149 us -> see profiles/r02_lossbench.txt), which stays for the A/B comparison.
+// in a fixed order.  No atomics anywhere: the gradient is bit-reproducible run to run; 4x fewer exponentials than one
+// warp per low-res cell gathering its whole footprint (124.7 -> 54.3 us at config 2, profiles/r02_lossbench.txt).
 // ------------------------------------------------------------------------------------------------
 template <int C, int NM>
 __global__ void __launch_bounds__(128) uvem_ce_grad_block_kernel(const float* __restrict__ x1, const float* __restrict__ x2, int b, int h,
@@ -439,38 +346,29 @@ extern "C" int uem_uvem_loss_forward_f32(const float* x1, const float* x2, int b
 }
 
 // g_m (b,c,h,w) = scale[0] * d/dx_m sum_px coef * CE(up(x_m))[target]; every element is written (no zero-init needed)
-// ws: uem_uvem_loss_backward_ws_bytes(b, c, h, w, heads) bytes of scratch (the per-block partials), or NULL for the
-// first form (one warp per low-res cell; 4x the exponentials, no scratch)
+// ws: uem_uvem_loss_backward_ws_bytes(b, c, h, w, heads) bytes of scratch (the per-block partials)
 extern "C" int uem_uvem_loss_backward_f32(const float* x1, const float* x2, int b, int c, int h, int w, int H, int W,
                                           const int64_t* target, const float* coef, const float* scale, float* g1, float* g2,
                                           void* ws, void* stream) {
     UEM_REQUIRE(x1 && g1 && target && coef && scale && b > 0 && h > 0 && w > 0 && H > 0 && W > 0,
                 "uem_uvem_loss_backward_f32: bad arguments");
     UEM_REQUIRE(!x2 == !g2, "uem_uvem_loss_backward_f32: second head needs its gradient buffer");
+    UEM_REQUIRE(ws, "uem_uvem_loss_backward_f32: ws is required (uem_uvem_loss_backward_ws_bytes bytes)");
     UEM_REQUIRE(h <= 65535 && b <= 65535, "uem_uvem_loss_backward_f32: grid too large");
     cudaStream_t st = (cudaStream_t)stream;
     const float sy = uem_align_corners_scale(h, H), sx = uem_align_corners_scale(w, W);
-    if (ws) {
-        const int64_t nblk = (int64_t)b * h * w;
-        const int64_t elems = nblk * c * (x2 ? 2 : 1);
-        const int ggrid = (int)min((int64_t)UEM_SMS * 8, (elems + 255) / 256);
-        UEM_DISPATCH_C(c, {
-            if (x2) {
-                uvem_ce_grad_block_kernel<C, 2><<<(unsigned)((nblk + 3) / 4), 128, 0, st>>>(x1, x2, b, h, w, H, W, sy, sx, target, coef, (float*)ws);
-                uvem_ce_grad_gather_kernel<C, 2><<<ggrid, 256, 0, st>>>((const float*)ws, b, h, w, scale, g1, g2);
-            } else {
-                uvem_ce_grad_block_kernel<C, 1><<<(unsigned)((nblk + 3) / 4), 128, 0, st>>>(x1, x2, b, h, w, H, W, sy, sx, target, coef, (float*)ws);
-                uvem_ce_grad_gather_kernel<C, 1><<<ggrid, 256, 0, st>>>((const float*)ws, b, h, w, scale, g1, g2);
-            }
-        });
-        UEM_CHECK_LAUNCH_N(2);
-        return 0;
-    }
-    dim3 grid(w, h, b);
+    const int64_t nblk = (int64_t)b * h * w;
+    const int64_t elems = nblk * c * (x2 ? 2 : 1);
+    const int ggrid = (int)min((int64_t)UEM_SMS * 8, (elems + 255) / 256);
     UEM_DISPATCH_C(c, {
-        if (x2) uvem_ce_grad_kernel<C, 2><<<grid, 32, 0, st>>>(x1, x2, h, w, H, W, sy, sx, target, coef, scale, g1, g2);
-        else uvem_ce_grad_kernel<C, 1><<<grid, 32, 0, st>>>(x1, x2, h, w, H, W, sy, sx, target, coef, scale, g1, g2);
+        if (x2) {
+            uvem_ce_grad_block_kernel<C, 2><<<(unsigned)((nblk + 3) / 4), 128, 0, st>>>(x1, x2, b, h, w, H, W, sy, sx, target, coef, (float*)ws);
+            uvem_ce_grad_gather_kernel<C, 2><<<ggrid, 256, 0, st>>>((const float*)ws, b, h, w, scale, g1, g2);
+        } else {
+            uvem_ce_grad_block_kernel<C, 1><<<(unsigned)((nblk + 3) / 4), 128, 0, st>>>(x1, x2, b, h, w, H, W, sy, sx, target, coef, (float*)ws);
+            uvem_ce_grad_gather_kernel<C, 1><<<ggrid, 256, 0, st>>>((const float*)ws, b, h, w, scale, g1, g2);
+        }
     });
-    UEM_CHECK_LAUNCH();
+    UEM_CHECK_LAUNCH_N(2);
     return 0;
 }

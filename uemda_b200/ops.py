@@ -494,9 +494,8 @@ def uvem_loss_forward(x1, x2, target, coef):
     return sums
 
 
-def uvem_loss_backward(x1, x2, target, coef, scale, per_cell=False):
-    """scale * d/dx_m sum_px coef * CE(upsample(x_m))[target]; deterministic (no atomics).  per_cell: the first form of the
-    kernel (one warp per low-res cell, every pixel's softmax evaluated by the 4 cells it touches), kept for A/B runs."""
+def uvem_loss_backward(x1, x2, target, coef, scale):
+    """scale * d/dx_m sum_px coef * CE(upsample(x_m))[target]; deterministic (no atomics)."""
     L.require_cuda(x1, x2, target, coef, scale)
     x1 = L.f32c(x1.detach())
     x2 = None if x2 is None else L.f32c(x2.detach())
@@ -508,7 +507,7 @@ def uvem_loss_backward(x1, x2, target, coef, scale, per_cell=False):
     lib = L.bind(x1)
     g1 = torch.empty_like(x1)
     g2 = None if x2 is None else torch.empty_like(x2)
-    ws = None if per_cell else L.workspace(lib.uem_uvem_loss_backward_ws_bytes(b, c, h, w, 2 if x2 is not None else 1), x1)
+    ws = L.workspace(lib.uem_uvem_loss_backward_ws_bytes(b, c, h, w, 2 if x2 is not None else 1), x1)
     L.check(lib.uem_uvem_loss_backward_f32(L.ptr(x1), L.ptr(x2), b, c, h, w, H, W, L.ptr(target), L.ptr(coef), L.ptr(scale),
                                            L.ptr(g1), L.ptr(g2), L.ptr(ws), L.stream_of(x1)))
     return g1, g2
