@@ -795,6 +795,31 @@ def test_region_phase_carries_the_id_send(dev, world):
                 _eq(a, b2, "rank %d staged %s" % (r, name))
 
 
+def test_refused_region_phase_sends_nothing_later(dev):
+    """8e: an id-carrying region phase that is refused (a region capacity past the shared-memory table) sends nothing,
+    and a plain region phase issued next on the same thread does not carry that send either: the exchange region stays
+    untouched and no poll times out."""
+    from uemda_b200 import mining
+    from uemda_b200.exchange import PeerExchange
+    from uemda_b200.synth import WORKLOADS, make_inputs
+    wl = WORKLOADS["tiny"]
+    (peer,) = PeerExchange.local_only(1, wl.c, wl.k, device=dev)
+    inp = _to(make_inputs(wl, seed=7), dev)
+    gid = torch.zeros(1, dtype=torch.int64, device=dev)
+    big = 20000
+    ws_big = mining.mine_workspace(inp["soft"], big, wl.h, wl.w, wl.k)
+    with pytest.raises(RuntimeError):
+        mining.region_phase(inp["soft"], inp["sup"], 2.0, big, ws_big, wl.h, wl.w, wl.k, exchange=(peer, 0, gid))
+    R = int(inp["ignore_id"]) + 1
+    ws = mining.mine_workspace(inp["soft"], R, wl.h, wl.w, wl.k)
+    local = mining.region_phase(inp["soft"], inp["sup"], 2.0, R, ws, wl.h, wl.w, wl.k)
+    assert int(local.item()) == int(inp["sup"].max().item())
+    region = peer._keep[peer.rank]
+    assert int(region.count_nonzero()) == 0, "the exchange region was written by a call that asked for no exchange"
+    assert int(gid.item()) == 0
+    assert peer.status() == 0
+
+
 def mining_down(inp, wl):
     from uemda_b200.gast.alignment import DownscaleLabel
     return DownscaleLabel(wl.scale, wl.c, -1, 0.75)(inp["label_s"])

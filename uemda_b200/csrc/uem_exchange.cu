@@ -23,6 +23,9 @@
 //                                bit-identical), local mean, keep-old rule, EMA; the last CTA acknowledges the slot to every
 //                                peer (one release store per peer), which is what a sender checks before it overwrites that
 //                                slot `depth` steps later.
+//   uem_xchg_exchange_fold_ema   the sums part of the send and the fold above in ONE launch.
+// Each protocol step (slot addressing, LL stores, acknowledgement wait, id poll, the receiving end) is written once in
+// uem_xchg_dev.cuh, and the fold / EMA arithmetic once in uem_proto_stats.cuh.
 // No kernel waits for a kernel that is queued behind it on its own GPU: a send of step s waits for the acks of step
 // s - depth, the consumers of step s for the sends of step s -- both are upstream in every rank's stream order, so the
 // scheme cannot deadlock however the ranks drift.  Every poll is bounded (2 s of %globaltimer): on a timeout status bit 8
@@ -50,69 +53,39 @@ __global__ void __launch_bounds__(256) xchg_send_kernel(const float* __restrict_
     // releases its dependents at entry): its CTAs are resident by the time that kernel ends, the launch latency is hidden
     asm volatile("griddepcontrol.wait;" ::: "memory");
     if (threadIdx.x == 0) {
-        const unsigned my = *reinterpret_cast<volatile unsigned*>(&hdr->seq_send[slot]) + 1u;
-        // peer p must have folded the previous contents of this slot (its ack lands in MY region)
-        const unsigned* ack = reinterpret_cast<const unsigned*>(mine + kOffAcks) + slot * kMaxWorld + p;
-        if (!spin_until(ack, my - 1u)) atomicOr(&hdr->status, 8);
-        s_my = my;
+        s_my = *reinterpret_cast<volatile unsigned*>(&hdr->seq_send[slot]) + 1u;
+        wait_ack(mine, slot, p, s_my);
     }
     __syncthreads();
     const unsigned my = s_my;
     const int ck = c * k;
-    const int64_t sb = slot_bytes(c, k);
-    char* dst = peers.base[p] + kOffSlots + ((int64_t)slot * world + rank) * sb;
-    // chunk ch of the sums, 4 floats at a time; per-image partials folded in image order (the same fp32 additions as
-    // proto_fold_kernel / proto_fold_finalize_kernel: a one-rank exchange reproduces the single-GPU step bit for bit)
+    char* dst = peers.base[p] + slot_off(slot, world, rank, c, k);
+    // chunk ch of the sums, 4 elements at a time, this rank's partials folded over its images
     const int nvec = (parts & 1) ? (ck + 3) / 4 : 0;   // parts bit 0: sums + counts + histogram; bit 1: max id
     const int v0 = (int)((int64_t)nvec * ch / gridDim.x), v1 = (int)((int64_t)nvec * (ch + 1) / gridDim.x);
     for (int v = v0 + threadIdx.x; v < v1; v += blockDim.x) {
-        float s[4] = {0.f, 0.f, 0.f, 0.f};
+        const int64_t e = (int64_t)4 * v;
         if ((ck & 3) == 0) {
-            for (int bi = 0; bi < b; ++bi) {
-                const float4 q = __ldg(reinterpret_cast<const float4*>(partial + (int64_t)bi * ck) + v);
-                s[0] += q.x; s[1] += q.y; s[2] += q.z; s[3] += q.w;
-            }
+            const float4 s = fold_images4(partial, b, ck, v);
+            ll_store(dst + e * 8, __float_as_uint(s.x), my);
+            ll_store(dst + e * 8 + 8, __float_as_uint(s.y), my);
+            ll_store(dst + e * 8 + 16, __float_as_uint(s.z), my);
+            ll_store(dst + e * 8 + 24, __float_as_uint(s.w), my);
         } else {
-            for (int bi = 0; bi < b; ++bi)
-#pragma unroll
-                for (int u = 0; u < 4; ++u)
-                    if (4 * v + u < ck) s[u] += partial[(int64_t)bi * ck + 4 * v + u];
+            for (int u = 0; u < 4; ++u)   // ragged last vector (ck % 4 != 0): zero words past the end
+                ll_store(dst + (e + u) * 8, __float_as_uint(e + u < ck ? fold_images(partial, b, ck, e + u) : 0.f), my);
         }
-#pragma unroll
-        for (int u = 0; u < 4; ++u) ll_store(dst + ((int64_t)4 * v + u) * 8, __float_as_uint(s[u]), my);
     }
     if (ch == 0 && threadIdx.x < 2 * c + 2 && ((threadIdx.x == 2 * c + 1) ? (parts & 2) : (parts & 1))) {
-        char* tail = dst + sum_words(c, k) * 8;
         const int i = threadIdx.x;
-        int64_t v;
-        if (i < c) {
-            v = 0;
-            for (int bi = 0; bi < b; ++bi) v += cnt_partial[bi * c + i];
-        } else if (i < 2 * c + 1) {
-            v = hist ? hist[i - c] : 0;
-        } else {
-            v = max_id ? max_id[0] : -1;
-        }
-        ll_store(tail + (int64_t)i * 16, (unsigned)((uint64_t)v & 0xffffffffu), my);
-        ll_store(tail + (int64_t)i * 16 + 8, (unsigned)((uint64_t)v >> 32), my);
+        const int64_t v = i < c ? fold_image_counts(cnt_partial, b, c, i) : (i < 2 * c + 1 ? (hist ? hist[i - c] : 0) : (max_id ? max_id[0] : -1));
+        ll_store_i64(dst + tail_off(c, k) + (int64_t)i * 16, v, my);
     }
     // optional: the CTA that fills this rank's own slot also polls the other ranks' max ids of the same step and leaves
     // the batch-global id (alignment.py:241) for the refine kernel of the NEXT graph -- no separate wait launch
     if (global_id_out && ch == 0 && p == rank && threadIdx.x < 32) {
-        const int r = threadIdx.x;
-        long long id = LLONG_MIN;
-        if (r < world) {
-            const char* src = mine + kOffSlots + ((int64_t)slot * world + r) * sb + sum_words(c, k) * 8 + (int64_t)(2 * c + 1) * 16;
-            bool ok = true;
-            id = ll_load_i64(src, my, &ok);
-            if (!ok) atomicOr(&hdr->status, 8);
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            const long long other = __shfl_xor_sync(0xffffffffu, id, o);
-            id = other > id ? other : id;
-        }
-        if (r == 0) global_id_out[0] = id;
+        const long long id = poll_max_id(mine, slot, world, c, k, my);
+        if (threadIdx.x == 0) global_id_out[0] = id;
     }
     // the last CTA of the FINAL launch of a step (parts bit 2) advances the local sequence number (every CTA has read it by
     // then); an earlier partial launch of the same step leaves it alone, so both tag their words with the same number
@@ -130,81 +103,27 @@ __global__ void __launch_bounds__(256) xchg_send_kernel(const float* __restrict_
 
 __global__ void __launch_bounds__(32) xchg_wait_maxid_kernel(char* __restrict__ region, int world, int slot, int c, int k,
                                                              int64_t* __restrict__ max_id_out) {
-    XHeader* hdr = reinterpret_cast<XHeader*>(region);
-    const unsigned want = *reinterpret_cast<volatile unsigned*>(&hdr->seq_recv[slot]) + 1u;
-    const int r = threadIdx.x;
-    long long id = LLONG_MIN;
-    if (r < world) {
-        const int64_t sb = slot_bytes(c, k);
-        const char* src = region + kOffSlots + ((int64_t)slot * world + r) * sb + sum_words(c, k) * 8 + (int64_t)(2 * c + 1) * 16;
-        bool ok = true;
-        id = ll_load_i64(src, want, &ok);
-        if (!ok) atomicOr(&hdr->status, 8);
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const long long other = __shfl_xor_sync(0xffffffffu, id, o);
-        id = other > id ? other : id;
-    }
-    if (r == 0 && max_id_out) max_id_out[0] = id;
+    const unsigned want = *reinterpret_cast<volatile unsigned*>(&reinterpret_cast<XHeader*>(region)->seq_recv[slot]) + 1u;
+    const long long id = poll_max_id(region, slot, world, c, k, want);
+    if (threadIdx.x == 0 && max_id_out) max_id_out[0] = id;
 }
 
 __global__ void __launch_bounds__(256) xchg_fold_finalize_kernel(const __grid_constant__ Peers peers, int rank, int world, int slot, int c, int k,
                                                                  const float* __restrict__ proto_old, float eps, float one_minus_decay,
                                                                  float decay, float* __restrict__ proto_new, float* __restrict__ sums_out,
                                                                  int64_t* __restrict__ counts_out, int64_t* __restrict__ hist_out) {
-    char* const region = peers.base[rank];
-    XHeader* hdr = reinterpret_cast<XHeader*>(region);
+    XHeader* hdr = reinterpret_cast<XHeader*>(peers.base[rank]);
     const unsigned want = *reinterpret_cast<volatile unsigned*>(&hdr->seq_recv[slot]) + 1u;
-    const int ck = c * k;
-    const int64_t sb = slot_bytes(c, k);
-    const char* slots = region + kOffSlots + (int64_t)slot * world * sb;
-    const char* tails = slots + sum_words(c, k) * 8;
-    const int i = blockIdx.x * 256 + threadIdx.x;
-    bool ok = true;
-    if (i < ck) {
-        const int ci = i / k;
-        float s;
-        int64_t n;
-        ll_fold_ranks(slots + (int64_t)i * 8, tails + (int64_t)ci * 16, sb, world, want, &s, &n, &ok);   // rank order: identical on every rank
-        if (sums_out) sums_out[i] = s;
-        if (proto_new) {
-            const float old = proto_old[i];
-            float local = s / ((float)n + eps);                 // alignment.py:348
-            if (n < 1) local = old;                             // :350
-            proto_new[i] = __fadd_rn(__fmul_rn(one_minus_decay, local), __fmul_rn(decay, old));   // :465
-        }
-    }
-    if (i < 2 * c + 1 && (counts_out || hist_out)) {
-        int64_t n = 0;
-        for (int r = 0; r < world; ++r) n += ll_load_i64(tails + r * sb + (int64_t)i * 16, want, &ok);
-        if (i < c) { if (counts_out) counts_out[i] = n; }
-        else if (hist_out) hist_out[i - c] = n;
-    }
-    if (!ok) atomicOr(&hdr->status, 8);
-    // the last CTA acknowledges the slot to every peer and advances the local sequence number
-    __threadfence();
-    __syncthreads();
-    __shared__ int s_last;
-    if (threadIdx.x == 0) s_last = (atomicAdd(&hdr->fold_arrive[slot], 1u) == gridDim.x - 1);
-    __syncthreads();
-    if (s_last) {
-        if (threadIdx.x < world)
-            st_release_sys(reinterpret_cast<unsigned*>(peers.base[threadIdx.x] + kOffAcks) + slot * kMaxWorld + rank, want);
-        if (threadIdx.x == 0) {
-            hdr->fold_arrive[slot] = 0u;
-            __threadfence();
-            *reinterpret_cast<volatile unsigned*>(&hdr->seq_recv[slot]) = want;
-        }
-    }
+    xchg_fold_ema_ack(peers, rank, world, slot, c, k, want, false, proto_old, eps, one_minus_decay, decay, proto_new, sums_out,
+                      counts_out, hist_out);
 }
 
 // ------------------------------------------------------------------------------------------------
-// One launch per step for the sums: local fold -> LL stores into every rank's slot -> poll every rank's words -> rank-ordered
-// fold -> keep-old rule -> EMA -> acknowledgement.  Thread i owns element i of the (c,k) bank from its own partials to the
-// new prototype; CTA 0 also carries the counts / histogram words.  (The max id travels earlier, uem_xchg_send_f32 with
-// parts = 2, tagged with the same sequence number.)  A CTA sends before it polls and its peers' CTAs do the same, so no
-// poll waits for anything that is queued behind this launch on any GPU.
+// One launch per step for the sums: local fold -> LL stores into every rank's slot -> the receiving end of
+// xchg_fold_finalize_kernel, which here also advances the send sequence number.  Thread i owns element i of the (c,k)
+// bank from its own partials to the new prototype; CTA 0 also carries the counts / histogram words.  (The max id travels
+// earlier, uem_xchg_send_f32 with parts = 2, tagged with the same sequence number.)  A CTA sends before it polls and its
+// peers' CTAs do the same, so no poll waits for anything that is queued behind this launch on any GPU.
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) xchg_exchange_fold_kernel(const float* __restrict__ partial, const int* __restrict__ cnt_partial,
                                                                  int b, int c, int k, const int64_t* __restrict__ hist, const __grid_constant__ Peers peers,
@@ -215,75 +134,25 @@ __global__ void __launch_bounds__(256) xchg_exchange_fold_kernel(const float* __
     char* const mine = peers.base[rank];
     XHeader* hdr = reinterpret_cast<XHeader*>(mine);
     __shared__ unsigned s_my;
-    __shared__ int s_last;
     if (threadIdx.x == 0) s_my = *reinterpret_cast<volatile unsigned*>(&hdr->seq_send[slot]) + 1u;
     __syncthreads();
     const unsigned my = s_my;
-    if (threadIdx.x < world) {   // every peer must have folded the previous contents of this slot
-        const unsigned* ack = reinterpret_cast<const unsigned*>(mine + kOffAcks) + slot * kMaxWorld + threadIdx.x;
-        if (!spin_until(ack, my - 1u)) atomicOr(&hdr->status, 8);
-    }
+    if (threadIdx.x < world) wait_ack(mine, slot, threadIdx.x, my);   // every peer must have folded the previous contents
     __syncthreads();
     const int ck = c * k;
-    const int64_t sb = slot_bytes(c, k);
-    const int64_t my_off = kOffSlots + ((int64_t)slot * world + rank) * sb;
+    const int64_t my_off = slot_off(slot, world, rank, c, k);
     const int i = blockIdx.x * 256 + threadIdx.x;
-    // ---- send: this rank's element i (per-image partials folded in image order) into every rank's slot
     if (i < ck) {
-        float s = 0.f;
-        for (int bi = 0; bi < b; ++bi) s += __ldg(partial + (int64_t)bi * ck + i);
+        const float s = fold_images(partial, b, ck, i);
         for (int p = 0; p < world; ++p) ll_store(peers.base[p] + my_off + (int64_t)i * 8, __float_as_uint(s), my);
     }
     if (blockIdx.x == 0 && threadIdx.x < 2 * c + 1) {
         const int t = threadIdx.x;
-        int64_t v = 0;
-        if (t < c) { for (int bi = 0; bi < b; ++bi) v += cnt_partial[bi * c + t]; }
-        else v = hist ? hist[t - c] : 0;
-        for (int p = 0; p < world; ++p) {
-            char* tail = peers.base[p] + my_off + sum_words(c, k) * 8 + (int64_t)t * 16;
-            ll_store(tail, (unsigned)((uint64_t)v & 0xffffffffu), my);
-            ll_store(tail + 8, (unsigned)((uint64_t)v >> 32), my);
-        }
+        const int64_t v = t < c ? fold_image_counts(cnt_partial, b, c, t) : (hist ? hist[t - c] : 0);
+        for (int p = 0; p < world; ++p) ll_store_i64(peers.base[p] + my_off + tail_off(c, k) + (int64_t)t * 16, v, my);
     }
-    // ---- receive + fold in rank order + EMA
-    const char* slots = mine + kOffSlots + (int64_t)slot * world * sb;
-    const char* tails = slots + sum_words(c, k) * 8;
-    bool ok = true;
-    if (i < ck) {
-        const int ci = i / k;
-        float s;
-        int64_t n;
-        ll_fold_ranks(slots + (int64_t)i * 8, tails + (int64_t)ci * 16, sb, world, my, &s, &n, &ok);   // rank order
-        if (sums_out) sums_out[i] = s;
-        if (proto_new) {
-            const float old = proto_old[i];
-            float local = s / ((float)n + eps);                 // alignment.py:348
-            if (n < 1) local = old;                             // :350
-            proto_new[i] = __fadd_rn(__fmul_rn(one_minus_decay, local), __fmul_rn(decay, old));   // :465
-        }
-    }
-    if (i < 2 * c + 1 && (counts_out || hist_out)) {
-        int64_t n = 0;
-        for (int r = 0; r < world; ++r) n += ll_load_i64(tails + r * sb + (int64_t)i * 16, my, &ok);
-        if (i < c) { if (counts_out) counts_out[i] = n; }
-        else if (hist_out) hist_out[i - c] = n;
-    }
-    if (!ok) atomicOr(&hdr->status, 8);
-    // ---- the last CTA acknowledges the slot to every peer and advances both sequence numbers
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) s_last = (atomicAdd(&hdr->fold_arrive[slot], 1u) == gridDim.x - 1);
-    __syncthreads();
-    if (s_last) {
-        if (threadIdx.x < world)
-            st_release_sys(reinterpret_cast<unsigned*>(peers.base[threadIdx.x] + kOffAcks) + slot * kMaxWorld + rank, my);
-        if (threadIdx.x == 0) {
-            hdr->fold_arrive[slot] = 0u;
-            __threadfence();
-            *reinterpret_cast<volatile unsigned*>(&hdr->seq_send[slot]) = my;
-            *reinterpret_cast<volatile unsigned*>(&hdr->seq_recv[slot]) = my;
-        }
-    }
+    xchg_fold_ema_ack(peers, rank, world, slot, c, k, my, true, proto_old, eps, one_minus_decay, decay, proto_new, sums_out,
+                      counts_out, hist_out);
 }
 
 }  // namespace
@@ -300,8 +169,7 @@ extern "C" int uem_xchg_send_f32(const void* partials_ws, int b, int c, int k, c
     UEM_REQUIRE(!(parts & 1) || partials_ws, "uem_xchg_send_f32: the sums part needs the partials");
     Peers P;
     if (int rc = fill_peers(&P, peer_regions, rank, world, depth, slot, "uem_xchg_send_f32")) return rc;
-    const float* partial = (const float*)partials_ws;
-    const int* cnt_partial = partial ? (const int*)(partial + (int64_t)b * c * k) : nullptr;
+    const ProtoPartials PP = proto_partials(partials_ws, b, c, k);
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((parts & 1) ? kSendChunks : 1, world, 1);
     cfg.blockDim = dim3(256, 1, 1);
@@ -311,7 +179,7 @@ extern "C" int uem_xchg_send_f32(const void* partials_ws, int b, int c, int k, c
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = (parts == 2) ? 1 : 0;   // id only: overlap the launch with the preceding (region-max) kernel
-    UEM_CUDA(cudaLaunchKernelEx(&cfg, xchg_send_kernel, partial, cnt_partial, b, c, k, max_id, hist, P, rank, world, slot, global_id_out, parts));
+    UEM_CUDA(cudaLaunchKernelEx(&cfg, xchg_send_kernel, PP.sums, PP.counts, b, c, k, max_id, hist, P, rank, world, slot, global_id_out, parts));
     UEM_CHECK_LAUNCH();
     return 0;
 }
@@ -344,10 +212,9 @@ extern "C" int uem_xchg_exchange_fold_ema_f32(const void* partials_ws, int b, in
                 "uem_xchg_exchange_fold_ema_f32: bad arguments");
     Peers P;
     if (int rc = fill_peers(&P, peer_regions, rank, world, depth, slot, "uem_xchg_exchange_fold_ema_f32")) return rc;
-    const float* partial = (const float*)partials_ws;
-    const int* cnt_partial = (const int*)(partial + (int64_t)b * c * k);
+    const ProtoPartials PP = proto_partials(partials_ws, b, c, k);
     xchg_exchange_fold_kernel<<<uem_div_up((int64_t)c * k, 256), 256, 0, (cudaStream_t)stream>>>(
-        partial, cnt_partial, b, c, k, hist, P, rank, world, slot, proto_old, eps, one_minus_decay, decay, proto_new, sums_out, counts_out,
+        PP.sums, PP.counts, b, c, k, hist, P, rank, world, slot, proto_old, eps, one_minus_decay, decay, proto_new, sums_out, counts_out,
         hist_out);
     UEM_CHECK_LAUNCH();
     return 0;

@@ -75,7 +75,7 @@ __device__ __forceinline__ Ring ring_carve(unsigned char* smem) {
     r.empty = r.full + kStages;
     return r;
 }
-constexpr size_t kRingBytes = (size_t)kStages * (kKT * kPT + kKT * kPS) * 4 + 2 * kStages * 8;
+constexpr size_t kTileRingBytes = (size_t)kStages * (kKT * kPT + kKT * kPS) * 4 + 2 * kStages * 8;
 
 // producer lane: feature tiles [kKT x kPT] + the matching rows of the (k,8) prototype table, one barrier per stage
 __device__ __forceinline__ void ring_produce(const Ring& r, const CUtensorMap* tmap, const float* ph, int k, int px0, int kbeg, int ntiles,
@@ -101,7 +101,7 @@ __global__ void __launch_bounds__(kThreads) pcl_forward_tma_kernel(const __grid_
     constexpr int NA = 1 + M;
     extern __shared__ __align__(128) unsigned char smem_f[];
     const Ring r = ring_carve(smem_f);
-    float* part = reinterpret_cast<float*>(smem_f + kRingBytes);  // [NA][kPT] CTA partial (cluster-visible)
+    float* part = reinterpret_cast<float*>(smem_f + kTileRingBytes);  // [NA][kPT] CTA partial (cluster-visible)
     cg::cluster_group cluster = cg::this_cluster();
     const int ks = (int)cluster.block_rank(), KS = (int)cluster.num_blocks();
     const int ptile = blockIdx.x / KS, bi = blockIdx.y;
@@ -332,7 +332,7 @@ extern "C" int uem_pcl_forward_f32(const float* feat, int b, int k, int64_t hw, 
     const int kper = ((k + KS - 1) / KS + kKT - 1) / kKT * kKT;
     UEM_DISPATCH_C(c, {
         pcl_prep_kernel<<<C + 1, 256, 0, st>>>(protos, C, k, labels, (int64_t)b * hw, ignore_label, ph, nvalid);
-        const size_t smem = kRingBytes + (size_t)kPT * (1 + C) * 4;
+        const size_t smem = kTileRingBytes + (size_t)kPT * (1 + C) * 4;
         UEM_CUDA(cudaFuncSetAttribute(pcl_forward_tma_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3(ptiles * KS, b, 1);
@@ -368,8 +368,8 @@ extern "C" int uem_pcl_backward_f32(const float* feat, int b, int k, int64_t hw,
     while (KS < 16 && (int64_t)ptiles * b * KS < 3 * UEM_SMS && k / (KS * 2) >= 4 * kKT) KS *= 2;
     const int kper = ((k + KS - 1) / KS + kKT - 1) / kKT * kKT;
     UEM_DISPATCH_C(c, {
-        UEM_CUDA(cudaFuncSetAttribute(pcl_backward_tma_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRingBytes));
-        pcl_backward_tma_kernel<C><<<dim3(ptiles, b, KS), kThreads, kRingBytes, st>>>(tmap, k, (int)hw, kper, ph, coef, grad_out, grad_feat);
+        UEM_CUDA(cudaFuncSetAttribute(pcl_backward_tma_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTileRingBytes));
+        pcl_backward_tma_kernel<C><<<dim3(ptiles, b, KS), kThreads, kTileRingBytes, st>>>(tmap, k, (int)hw, kper, ph, coef, grad_out, grad_feat);
     });
     UEM_CHECK_LAUNCH();
     return 0;

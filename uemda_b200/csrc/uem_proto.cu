@@ -5,10 +5,11 @@
 //
 // The reference builds one-hot tensors ((b,c+1,H,W) f32, (n,c) int64) and an (n,c,k) broadcast product
 // (403 MB at config 2).  Here: DownscaleLabel is one pass over the int64 label map with per-thread
-// register bins; the prototype sums read the NCHW feature map exactly once (one warp per (image,
-// channel) row, 128-bit loads, class ids staged as bytes in shared memory, c register accumulators)
-// and are combined over the batch in a fixed order, so results are bit-reproducible run to run.
-#include "uem_common.cuh"
+// register bins; the prototype sums read the NCHW feature map exactly once (TMA tiles and one-hot
+// class planes when hw % 4 == 0, otherwise one warp per (image, channel rows) with the class ids staged
+// as bytes in shared memory) into per-image partials, which every consumer folds over the batch in
+// image order with the helpers of uem_proto_stats.cuh, so results are bit-reproducible run to run.
+#include "uem_proto_stats.cuh"
 #include "uem_tma.cuh"
 
 #ifndef UEM_PROTO_RW
@@ -229,114 +230,6 @@ __global__ void __launch_bounds__(kAccThreads) proto_accum_kernel(const float* _
     }
 }
 
-// 128-bit path of the masked class sums, built for bytes in flight and few instructions:
-//   * the class ids of a pixel tile become C one-hot fp32 planes in shared memory (mask[c][px]);
-//   * every warp streams kChPerWarp channel rows through a per-thread cp.async ring (kRing steps x kChPerWarp
-//     x 16 B = 256 B in flight per thread, no staging registers);
-//   * sums use packed FFMA2 over pixel pairs: acc2[q][c] += (m.x,m.y)*(v.x,v.y) ; += (m.z,m.w)*(v.z,v.w)
-//     = 2 instructions per (channel, class, 4 pixels) instead of 12 compare/select/add.
-constexpr int kRing = 4;
-constexpr int kMaskTile = 2048;  // pixels per mask tile (C*8 KB of shared memory)
-
-template <int C>
-__global__ void __launch_bounds__(kAccThreads, 2) proto_accum_ring_kernel(const float* __restrict__ feat, int k, int64_t hw,
-                                                                          const int64_t* __restrict__ label, int64_t ignore_label,
-                                                                          int tile_px, float* __restrict__ partial,
-                                                                          int* __restrict__ cnt_partial) {
-    extern __shared__ __align__(16) unsigned char smem_acc[];
-    float* mask = reinterpret_cast<float*>(smem_acc);                                 // [C][tile_px]
-    float4* ring = reinterpret_cast<float4*>(mask + (size_t)C * tile_px);             // [kRing][kChPerWarp][kAccThreads]
-    const int bi = blockIdx.y;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int kk0 = (blockIdx.x * (kAccThreads / 32) + warp) * kChPerWarp;
-    const float* f = feat + ((int64_t)bi * k + kk0) * hw;
-    const int64_t* lab = label + (int64_t)bi * hw;
-
-    float2 acc2[kChPerWarp][C];
-#pragma unroll
-    for (int q = 0; q < kChPerWarp; ++q)
-#pragma unroll
-        for (int ci = 0; ci < C; ++ci) acc2[q][ci] = make_float2(0.f, 0.f);
-    int cnt[C];
-#pragma unroll
-    for (int ci = 0; ci < C; ++ci) cnt[ci] = 0;
-
-    for (int64_t t0 = 0; t0 < hw; t0 += tile_px) {
-        const int tp = (int)min((int64_t)tile_px, hw - t0);
-        __syncthreads();
-        for (int i = threadIdx.x; i < tp; i += kAccThreads) {
-            const int64_t l = lab[t0 + i];
-#pragma unroll
-            for (int ci = 0; ci < C; ++ci) {
-                const bool hit = (l == ci) && (l != ignore_label);
-                mask[ci * tile_px + i] = hit ? 1.0f : 0.0f;
-                cnt[ci] += hit;
-            }
-        }
-        __syncthreads();
-        const int groups = tp / 4;
-        const int n_steps = (groups + 31) / 32;
-        auto issue = [&](int step) {
-            const int g = step * 32 + lane;
-            if (step < n_steps && g < groups) {
-#pragma unroll
-                for (int q = 0; q < kChPerWarp; ++q)
-                    if (kk0 + q < k)
-                        cp_async_16(&ring[((step % kRing) * kChPerWarp + q) * kAccThreads + threadIdx.x], f + (int64_t)q * hw + t0 + 4 * g);
-            }
-            cp_async_commit_group();
-        };
-#pragma unroll
-        for (int d = 0; d < kRing; ++d) issue(d);
-        for (int stp = 0; stp < n_steps; ++stp) {
-            cp_async_wait_group<kRing - 1>();
-            const int g = stp * 32 + lane;
-            if (g < groups) {
-                float4 m[C];
-#pragma unroll
-                for (int ci = 0; ci < C; ++ci) m[ci] = *reinterpret_cast<const float4*>(mask + ci * tile_px + 4 * g);
-#pragma unroll
-                for (int q = 0; q < kChPerWarp; ++q) {
-                    if (kk0 + q < k) {
-                        const float4 v = ring[((stp % kRing) * kChPerWarp + q) * kAccThreads + threadIdx.x];
-                        const float2 v01 = make_float2(v.x, v.y), v23 = make_float2(v.z, v.w);
-#pragma unroll
-                        for (int ci = 0; ci < C; ++ci) {
-                            acc2[q][ci] = __ffma2_rn(make_float2(m[ci].x, m[ci].y), v01, acc2[q][ci]);
-                            acc2[q][ci] = __ffma2_rn(make_float2(m[ci].z, m[ci].w), v23, acc2[q][ci]);
-                        }
-                    }
-                }
-            }
-            issue(stp + kRing);
-        }
-        cp_async_wait_group<0>();
-    }
-#pragma unroll
-    for (int q = 0; q < kChPerWarp; ++q) {
-        if (kk0 + q >= k) break;
-#pragma unroll
-        for (int ci = 0; ci < C; ++ci) {
-            const float x = warp_sum(acc2[q][ci].x + acc2[q][ci].y);
-            if (lane == 0) partial[((int64_t)bi * C + ci) * k + kk0 + q] = x;
-        }
-    }
-    if (blockIdx.x == 0) {  // class counts of this image, once
-        __shared__ int scnt[kAccThreads / 32][C];
-#pragma unroll
-        for (int ci = 0; ci < C; ++ci) {
-            const int n = __reduce_add_sync(0xffffffffu, cnt[ci]);
-            if (lane == 0) scnt[warp][ci] = n;
-        }
-        __syncthreads();
-        if (threadIdx.x < C) {
-            int n = 0;
-            for (int i = 0; i < kAccThreads / 32; ++i) n += scnt[i][threadIdx.x];
-            cnt_partial[bi * C + threadIdx.x] = n;
-        }
-    }
-}
-
 // ------------------------------------------------------------------------------------------------
 // TMA form of the masked class sums (hw % 4 == 0): persistent CTAs loop over (image, block of 8*RW channels) items
 // and stream each item's [8*RW channels x 128 pixels] tiles (cp.async.bulk.tensor) through an mbarrier ring.
@@ -521,20 +414,12 @@ __global__ void __launch_bounds__(kAccThreads) proto_accum_soft_kernel(const flo
     }
 }
 
-// fold the per-image partials in image order (deterministic)
+// fold the per-image partials (sums; counts when both are given)
 __global__ void __launch_bounds__(256) proto_fold_kernel(const float* __restrict__ partial, const int* __restrict__ cnt_partial,
                                                          int b, int ck, int c, float* __restrict__ sums, int64_t* __restrict__ counts) {
     const int i = blockIdx.x * 256 + threadIdx.x;
-    if (i < ck) {
-        float s = 0.f;
-        for (int bi = 0; bi < b; ++bi) s += partial[(int64_t)bi * ck + i];
-        sums[i] = s;
-    }
-    if (counts && cnt_partial && i < c) {
-        int64_t n = 0;
-        for (int bi = 0; bi < b; ++bi) n += cnt_partial[bi * c + i];
-        counts[i] = n;
-    }
+    if (i < ck) sums[i] = fold_images(partial, b, ck, i);
+    if (counts && cnt_partial && i < c) counts[i] = fold_image_counts(cnt_partial, b, c, i);
 }
 
 __global__ void __launch_bounds__(256) proto_finalize_kernel(const float* __restrict__ sums, const int64_t* __restrict__ counts,
@@ -543,38 +428,22 @@ __global__ void __launch_bounds__(256) proto_finalize_kernel(const float* __rest
                                                              float* __restrict__ local_out, float* __restrict__ proto_new) {
     const int i = blockIdx.x * 256 + threadIdx.x;
     if (i >= c * k) return;
-    const int ci = i / k;
-    float local;
-    if (counts) {
-        const int64_t n = counts[ci];
-        local = sums[i] / ((float)n + eps);                 // alignment.py:348
-        if (n < 1) local = proto_old[i];                    // :350 classes without samples keep the old prototype
-    } else {
-        local = sums[i] / (float)mean_n;                    // torch.mean over n pixels, alignment.py:104
-    }
+    const float old = proto_old[i];
+    const float local = counts ? proto_local(sums[i], counts[i / k], old, eps)
+                               : sums[i] / (float)mean_n;   // torch.mean over n pixels, alignment.py:104
     if (local_out) local_out[i] = local;
-    if (proto_new)                                          // _ema, alignment.py:465: two rounded products, one rounded sum
-        proto_new[i] = __fadd_rn(__fmul_rn(one_minus_decay, local), __fmul_rn(decay, proto_old[i]));
+    if (proto_new) proto_new[i] = proto_ema_of(local, old, one_minus_decay, decay);
 }
 
-// fold of the per-image partials (image order, deterministic) + local mean + keep-old rule + EMA in ONE launch
-// (alignment.py:347-353, :463-466): the single-GPU step needs neither the folded sums nor a separate fold kernel
+// fold of the per-image partials + local mean + keep-old rule + EMA in ONE launch: the single-GPU step needs neither the
+// folded sums nor a separate fold kernel
 __global__ void __launch_bounds__(256) proto_fold_finalize_kernel(const float* __restrict__ partial, const int* __restrict__ cnt_partial,
                                                                   int b, int c, int k, const float* __restrict__ proto_old, float eps,
                                                                   float one_minus_decay, float decay, float* __restrict__ proto_new) {
     const int i = blockIdx.x * 256 + threadIdx.x;
     if (i >= c * k) return;
-    const int ci = i / k;
-    float s = 0.f;
-    int64_t n = 0;
-    for (int bi = 0; bi < b; ++bi) {
-        s += partial[(int64_t)bi * c * k + i];
-        n += cnt_partial[bi * c + ci];
-    }
-    const float old = proto_old[i];
-    float local = s / ((float)n + eps);
-    if (n < 1) local = old;
-    proto_new[i] = __fadd_rn(__fmul_rn(one_minus_decay, local), __fmul_rn(decay, old));
+    proto_new[i] = proto_ema(fold_images(partial, b, (int64_t)c * k, i), fold_image_counts(cnt_partial, b, c, i / k), proto_old[i], eps,
+                             one_minus_decay, decay);
 }
 
 }  // namespace
@@ -631,12 +500,10 @@ extern "C" int uem_proto_accum_nchw_f32(const float* feat, int b, int k, int64_t
     UEM_REQUIRE(hw <= 200 * 1024, "uem_proto_accum_nchw_f32: %lld feature pixels per image exceed the shared-memory label stage", (long long)hw);
     cudaStream_t st = (cudaStream_t)stream;
     float* partial = (float*)ws;
-    int* cnt_partial = (int*)(partial + (int64_t)b * c * k);
+    int* cnt_partial = (int*)proto_partials(ws, b, c, k).counts;
     const bool vec = (hw % 4 == 0) && uem_aligned16(feat);
-    const size_t smem = (size_t)((hw + 15) / 16) * 16;
     UEM_DISPATCH_C(c, {
-        dim3 grid(uem_div_up(k, (kAccThreads / 32) * kChPerWarp), b);
-        if (vec && hw < (1 << 30)) {
+        if (vec) {   // TMA form (hw fits int: at most 200K pixels)
             using P = ProtoTma<C, UEM_PROTO_RW>;
             CUtensorMap tmap;
             UEM_REQUIRE(uem_make_tmap_3d_f32(&tmap, feat, (uint64_t)hw, (uint64_t)k, (uint64_t)b, (uint64_t)hw, (uint64_t)k * hw, kTilePx,
@@ -651,12 +518,9 @@ extern "C" int uem_proto_accum_nchw_f32(const float* feat, int b, int k, int64_t
             const int nblk = min(total, UEM_SMS * per_sm);
             proto_accum_tma_kernel<C, UEM_PROTO_RW><<<nblk, kTmaThreads, P::SMEM, st>>>(tmap, k, (int)hw, b, label, ignore_label, partial,
                                                                                          cnt_partial, g_uem_l2_stream ? 1 : 0);
-        } else if (vec) {
-            const int tile_px = (int)min((int64_t)kMaskTile, ((hw + 3) / 4) * 4);
-            const size_t smem_r = (size_t)C * tile_px * 4 + (size_t)kRing * kChPerWarp * kAccThreads * 16;
-            UEM_CUDA(cudaFuncSetAttribute(proto_accum_ring_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_r));
-            proto_accum_ring_kernel<C><<<grid, kAccThreads, smem_r, st>>>(feat, k, hw, label, ignore_label, tile_px, partial, cnt_partial);
         } else {
+            const dim3 grid(uem_div_up(k, (kAccThreads / 32) * kChPerWarp), b);
+            const size_t smem = (size_t)((hw + 15) / 16) * 16;
             if (smem > 48 * 1024) UEM_CUDA(cudaFuncSetAttribute(proto_accum_kernel<C, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             proto_accum_kernel<C, 1><<<grid, kAccThreads, smem, st>>>(feat, k, hw, label, ignore_label, partial, cnt_partial);
         }
@@ -669,9 +533,8 @@ extern "C" int uem_proto_accum_nchw_f32(const float* feat, int b, int k, int64_t
 extern "C" int uem_proto_fold_finalize_ema_f32(const void* ws, int b, int c, int k, const float* proto_old, float eps,
                                                float one_minus_decay, float decay, float* proto_new, void* stream) {
     UEM_REQUIRE(ws && proto_old && proto_new && b > 0 && c > 0 && k > 0, "uem_proto_fold_finalize_ema_f32: bad arguments");
-    const float* partial = (const float*)ws;
-    const int* cnt_partial = (const int*)(partial + (int64_t)b * c * k);
-    proto_fold_finalize_kernel<<<uem_div_up((int64_t)c * k, 256), 256, 0, (cudaStream_t)stream>>>(partial, cnt_partial, b, c, k, proto_old, eps,
+    const ProtoPartials P = proto_partials(ws, b, c, k);
+    proto_fold_finalize_kernel<<<uem_div_up((int64_t)c * k, 256), 256, 0, (cudaStream_t)stream>>>(P.sums, P.counts, b, c, k, proto_old, eps,
                                                                                                 one_minus_decay, decay, proto_new);
     UEM_CHECK_LAUNCH();
     return 0;
@@ -743,35 +606,23 @@ __global__ void __launch_bounds__(256) fold_gathered_kernel(const double* __rest
 }  // namespace
 
 namespace {
-// per-image partials of proto_accumulate folded in image order (the same fp32 additions as proto_fold_kernel) and
-// packed in the same launch
+// per-image partials of proto_accumulate folded and packed in the same launch
 __global__ void __launch_bounds__(256) pack_partials_kernel(const float* __restrict__ partial, const int* __restrict__ cnt_partial,
                                                             const int64_t* __restrict__ max_id, int b, int ck, int c,
                                                             double* __restrict__ out) {
     const int n = ck + c + 1;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        if (i < ck) {
-            float s = 0.f;
-            for (int bi = 0; bi < b; ++bi) s += partial[(int64_t)bi * ck + i];
-            out[i] = (double)s;
-        } else if (i < ck + c) {
-            int64_t cnt = 0;
-            for (int bi = 0; bi < b; ++bi) cnt += cnt_partial[bi * c + (i - ck)];
-            out[i] = (double)cnt;
-        } else {
-            out[i] = (double)max_id[0];
-        }
-    }
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+        out[i] = i < ck ? (double)fold_images(partial, b, ck, i)
+                        : (i < ck + c ? (double)fold_image_counts(cnt_partial, b, c, i - ck) : (double)max_id[0]);
 }
 }  // namespace
 
 // ws: the per-image partials uem_proto_accum_nchw_f32 leaves when called with sums == NULL
 extern "C" int uem_pack_local_partials_f64(const void* ws, int b, int c, int k, const int64_t* max_id, double* out, void* stream) {
     UEM_REQUIRE(ws && max_id && out && b > 0 && c > 0 && k > 0, "uem_pack_local_partials_f64: bad arguments");
-    const float* partial = (const float*)ws;
-    const int* cnt_partial = (const int*)(partial + (int64_t)b * c * k);
+    const ProtoPartials P = proto_partials(ws, b, c, k);
     const int n = c * k + c + 1;
-    pack_partials_kernel<<<min(uem_div_up(n, 256), UEM_SMS), 256, 0, (cudaStream_t)stream>>>(partial, cnt_partial, max_id, b, c * k, c, out);
+    pack_partials_kernel<<<min(uem_div_up(n, 256), UEM_SMS), 256, 0, (cudaStream_t)stream>>>(P.sums, P.counts, max_id, b, c * k, c, out);
     UEM_CHECK_LAUNCH();
     return 0;
 }

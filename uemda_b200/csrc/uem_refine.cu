@@ -21,8 +21,8 @@
 // on (image, region): softmax(/temp)/max of the region maxima is precomputed per region (by the region-max kernel's tail
 // on the fused chain), the pixel kernels gather 2 x LDG.128; per-(image,class) maxima for pseudo_selection
 // (pseudo_generation.py:76) fall out as a (b, c+2) stats table raised with atomicMax.
-#include "uem_common.cuh"
 #include "uem_tma.cuh"
+#include "uem_xchg_dev.cuh"
 #include <string.h>
 
 int uem_region_table_f32(const float* src, int64_t sb, int64_t sn, int64_t sc, const int64_t* index, int b, int64_t N,
@@ -31,8 +31,7 @@ int uem_region_table_f32(const float* src, int64_t sb, int64_t sn, int64_t sc, c
 int uem_i64_max_accumulate(const int64_t* x, int64_t n, int64_t* out_max, cudaStream_t st);
 int uem_region_max_f32(const float* src, int64_t sb, int64_t sc, const int64_t* index, int b, int64_t N, int c, int64_t R,
                        unsigned* table, int64_t* maxid_out, int* status, float* tail_sw, int* tail_done, float temp,
-                       unsigned* zero_words, int n_zero, cudaStream_t st);
-int uem_region_arm_xchg(const void* const* peer_regions, int rank, int world, int depth, int slot, int c, int k, int64_t* global_id_out);
+                       unsigned* zero_words, int n_zero, const RegionXchg* xchg, cudaStream_t st);
 int uem_select_entropy_stats_impl(const float* mask, const uint32_t* class_stats, int b, int c, int64_t hw, float cutoff_top,
                                   float cutoff_low, int64_t ignore_label, int64_t* out, const float* uvem, float* entropy,
                                   float* weight, int64_t* zero_after, int pdl, cudaStream_t st);
@@ -1031,9 +1030,10 @@ static bool mine_selfclean(int views, int c, int64_t R) {
 // superpixel-view weights, and the rank-LOCAL max superpixel id at byte offset uem_mine_ws_maxid_offset(...) of ws.
 // The batch-global id (all-gather / all-reduce MAX across ranks, alignment.py:241) is only needed by the refine kernel,
 // so this half can run one step ahead of the exchange; uem_mine_refine_select_f32 with UEM_VIEW_REGIONS_READY then skips
-// it.  Same workspace, same self-cleaning protocol (the selection kernel zeroes the max-id slot again).
-extern "C" int uem_mine_region_phase_f32(const int64_t* sup, int64_t R, const float* soft, int b, int c, int H, int W, int h,
-                                         int w, int k, float temp, void* ws, void* stream) {
+// it.  Same workspace, same self-cleaning protocol (the selection kernel zeroes the max-id slot again).  xchg: the id
+// part of the step's multi-GPU send carried by the region-max kernel's last CTA, or nullptr.
+static int mine_region_phase(const int64_t* sup, int64_t R, const float* soft, int b, int c, int H, int W, int h, int w, int k,
+                             float temp, void* ws, const RegionXchg* xchg, void* stream) {
     UEM_REQUIRE(ws && soft && sup && b > 0 && H > 0 && W > 0, "uem_mine_region_phase_f32: bad arguments");
     UEM_REQUIRE(mine_selfclean(UEM_VIEW_SUP, c, R), "uem_mine_region_phase_f32: region capacity %lld does not fit the shared-memory table",
                 (long long)R);
@@ -1042,7 +1042,12 @@ extern "C" int uem_mine_region_phase_f32(const int64_t* sup, int64_t R, const fl
     const int64_t HW = (int64_t)H * W;
     return uem_region_max_f32(soft, (int64_t)c * HW, HW, sup, b, HW, c, R, (unsigned*)(base + L.region), (int64_t*)(base + L.maxid),
                               (int*)base, (float*)(base + L.sw), (int*)(base + L.done), temp, (unsigned*)(base + L.stats), b * (c + 2),
-                              (cudaStream_t)stream);
+                              xchg, (cudaStream_t)stream);
+}
+
+extern "C" int uem_mine_region_phase_f32(const int64_t* sup, int64_t R, const float* soft, int b, int c, int H, int W, int h,
+                                         int w, int k, float temp, void* ws, void* stream) {
+    return mine_region_phase(sup, R, soft, b, c, H, W, h, w, k, temp, ws, nullptr, stream);
 }
 
 // Same, and the LAST CTA of the region-max kernel also carries the id part of the step's multi-GPU send (uem_exchange.cu):
@@ -1052,8 +1057,11 @@ extern "C" int uem_mine_region_phase_xchg_f32(const int64_t* sup, int64_t R, con
                                               int w, int k, float temp, void* ws, const void* const* peer_regions, int rank, int world,
                                               int depth, int slot, int64_t* global_id_out, void* stream) {
     UEM_REQUIRE(c > 0 && k > 0, "uem_mine_region_phase_xchg_f32: bad arguments");
-    if (int rc = uem_region_arm_xchg(peer_regions, rank, world, depth, slot, c, k, global_id_out)) return rc;
-    return uem_mine_region_phase_f32(sup, R, soft, b, c, H, W, h, w, k, temp, ws, stream);
+    RegionXchg x{};
+    if (int rc = fill_peers(&x.peers, peer_regions, rank, world, depth, slot, "uem_mine_region_phase_xchg_f32")) return rc;
+    x.rank = rank; x.world = world; x.slot = slot; x.c = c; x.k = k;
+    x.global_id_out = (long long*)global_id_out;
+    return mine_region_phase(sup, R, soft, b, c, H, W, h, w, k, temp, ws, &x, stream);
 }
 
 extern "C" int uem_mine_proto_phase_f32(const float* feat, int k, const float* protos, int b, int c, int H, int W, int h, int w,
@@ -1149,7 +1157,7 @@ extern "C" int uem_mine_refine_select_f32(int views, const float* feat, int k, c
         // of the same pass when the caller did not supply it
         if (selfclean) {
             if ((rc = uem_region_max_f32(soft, (int64_t)c * HW, HW, sup, b, HW, c, R, table, own_maxid ? maxid : nullptr, status, sw,
-                                         (int*)(base + L.done), temp, stats, b * (c + 2), st)))
+                                         (int*)(base + L.done), temp, stats, b * (c + 2), nullptr, st)))
                 return rc;
             if (own_maxid) ignored_id = maxid;
         } else {

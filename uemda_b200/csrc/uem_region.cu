@@ -648,25 +648,13 @@ extern "C" int64_t uem_region_reduce_ws_bytes(int b, int64_t R, int c) {
     return ((int64_t)b * R * c + (int64_t)b * R + 4) * 4;
 }
 
-// The id part of a multi-GPU send armed for the NEXT fused region-max launch of this host thread (uem_mine_region_phase_xchg_f32).
-static thread_local RegionXchg g_armed_xchg;
-static thread_local bool g_has_armed_xchg = false;
-int uem_region_arm_xchg(const void* const* peer_regions, int rank, int world, int depth, int slot, int c, int k, int64_t* global_id_out) {
-    RegionXchg x{};
-    if (int rc = fill_peers(&x.peers, peer_regions, rank, world, depth, slot, "uem_mine_region_phase_xchg_f32")) return rc;
-    x.rank = rank; x.world = world; x.slot = slot; x.c = c; x.k = k;
-    x.global_id_out = (long long*)global_id_out;
-    g_armed_xchg = x;
-    g_has_armed_xchg = true;
-    return 0;
-}
-
 // Region maxima of a planar map into the encoded table (zero on entry); optionally the batch max id (maxid_out zero on
-// entry, ids are >= 0) and the fused weight tail (see RegionTail; tail_sw == nullptr: plain reduction).
+// entry, ids are >= 0), the fused weight tail (see RegionTail; tail_sw == nullptr: plain reduction) and, on the fused
+// chain, the id part of a multi-GPU send from the last CTA (xchg == nullptr: no send).
 // Needs R*c*4 + R bytes of shared memory per CTA.
 int uem_region_max_f32(const float* src, int64_t sb, int64_t sc, const int64_t* index, int b, int64_t N, int c, int64_t R,
                        unsigned* table, int64_t* maxid_out, int* status, float* tail_sw, int* tail_done, float temp,
-                       unsigned* zero_words, int n_zero, cudaStream_t st) {
+                       unsigned* zero_words, int n_zero, const RegionXchg* xchg, cudaStream_t st) {
     const bool vec = (N % 4 == 0) && (sb % 4 == 0) && (sc % 4 == 0) && uem_aligned16(src) && uem_aligned16(index);
     const size_t smem = ((size_t)R * ((c + 3) & ~3) * 4 + (size_t)((R + 3) / 4) * 4 + 15) & ~(size_t)15;
     UEM_REQUIRE(smem <= 200 * 1024, "uem_region_max_f32: region table (%lld x %d) exceeds shared memory", (long long)R, c);
@@ -678,12 +666,8 @@ int uem_region_max_f32(const float* src, int64_t sb, int64_t sc, const int64_t* 
     int chunks = max(1, (UEM_SMS * per_sm) / b);
     const int64_t groups = N / (vec ? 4 : 1);
     chunks = (int)min((int64_t)chunks, max((int64_t)1, groups / threads));
-    RegionXchg xchg{};
-    if (g_has_armed_xchg) {
-        g_has_armed_xchg = false;
-        UEM_REQUIRE(tail_sw && maxid_out, "uem_region_max_f32: the id send rides on the fused chain's region pass only");
-        xchg = g_armed_xchg;
-    }
+    UEM_REQUIRE(!xchg || (tail_sw && maxid_out), "uem_region_max_f32: the id send rides on the fused chain's region pass only");
+    const RegionXchg send = xchg ? *xchg : RegionXchg{};
     RegionTail tail{};
     tail.sw = tail_sw;
     tail.done = tail_done;
@@ -697,10 +681,10 @@ int uem_region_max_f32(const float* src, int64_t sb, int64_t sc, const int64_t* 
         dim3 grid(chunks, b);
         if (vec) {
             if (smem > 48 * 1024) UEM_CUDA(cudaFuncSetAttribute(region_max_smem_kernel<C, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            region_max_smem_kernel<C, 4><<<grid, threads, smem, st>>>(src, sb, sc, index, N, R, table, (long long*)maxid_out, status, tail, tail_sw ? g_uem_l2_region : 0, xchg);
+            region_max_smem_kernel<C, 4><<<grid, threads, smem, st>>>(src, sb, sc, index, N, R, table, (long long*)maxid_out, status, tail, tail_sw ? g_uem_l2_region : 0, send);
         } else {
             if (smem > 48 * 1024) UEM_CUDA(cudaFuncSetAttribute(region_max_smem_kernel<C, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            region_max_smem_kernel<C, 1><<<grid, threads, smem, st>>>(src, sb, sc, index, N, R, table, (long long*)maxid_out, status, tail, tail_sw ? g_uem_l2_region : 0, xchg);
+            region_max_smem_kernel<C, 1><<<grid, threads, smem, st>>>(src, sb, sc, index, N, R, table, (long long*)maxid_out, status, tail, tail_sw ? g_uem_l2_region : 0, send);
         }
     });
     UEM_CHECK_LAUNCH();
@@ -714,7 +698,7 @@ int uem_region_table_f32(const float* src, int64_t sb, int64_t sn, int64_t sc, c
     const int kop = (op == UEM_REDUCE_MAX) ? UEM_REDUCE_MAX : UEM_REDUCE_SUM;
     const bool vec = (sn == 1) && (N % 4 == 0) && (sb % 4 == 0) && (sc % 4 == 0) && uem_aligned16(src) && uem_aligned16(index);
     if (kop == UEM_REDUCE_MAX && !cnt && sn == 1 && R * (((c + 3) & ~3) * 4 + 1) + 64 <= 200 * 1024)
-        return uem_region_max_f32(src, sb, sc, index, b, N, c, R, table, nullptr, status, nullptr, nullptr, 1.0f, nullptr, 0, st);
+        return uem_region_max_f32(src, sb, sc, index, b, N, c, R, table, nullptr, status, nullptr, nullptr, 1.0f, nullptr, 0, nullptr, st);
     UEM_DISPATCH_C(c, {
         if (vec) {
             dim3 grid(uem_div_up(N / 4, kThreads * kSteps), b);

@@ -154,20 +154,9 @@ class PeerExchange:
     def fold_finalize(self, slot, proto_old=None, eps=1e-7, decay=None, out=None, want_sums=False, want_hist=False):
         """After ``wait_max_id`` on the same stream: rank-ordered fold (+ keep-old rule + EMA when ``decay`` is given; ``out``
         may be ``proto_old``) and the acknowledgement of the slot.  Returns (proto_new|None, sums|None, counts|None, hist|None)."""
-        dev = self.device
-        new = sums = counts = hist = None
-        omd = d = 0.0
-        if decay is not None:
-            proto_old = L.f32c(proto_old.detach())
-            new = out if out is not None else torch.empty_like(proto_old)
-            omd, d = ops.f32(1.0 - decay), ops.f32(decay)
-        if want_sums:
-            sums = torch.empty((self.c, self.k), dtype=torch.float32, device=dev)
-            counts = torch.empty((self.c,), dtype=torch.int64, device=dev)
-        if want_hist:
-            hist = torch.empty((self.c + 1,), dtype=torch.int64, device=dev)
+        proto_old, new, omd, d, sums, counts, hist = self._fold_outputs(proto_old, decay, out, want_sums, want_hist)
         lib = L.load()
-        stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        stream = ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
         L.check(lib.uem_xchg_fold_finalize_ema_f32(self._arr, self.rank, self.world, self.depth, int(slot), self.c, self.k,
                                                    L.ptr(proto_old), ops.f32(eps), omd, d, L.ptr(new), L.ptr(sums), L.ptr(counts),
                                                    L.ptr(hist), stream))
@@ -180,8 +169,18 @@ class PeerExchange:
         ws, (b, c, k) = partials
         assert (c, k) == (self.c, self.k)
         L.require_cuda(ws, hist, proto_old)
+        proto_old, new, omd, d, sums, counts, hist_out = self._fold_outputs(proto_old, decay, out, want_sums, want_hist)
+        lib = L.bind(ws)
+        L.check(lib.uem_xchg_exchange_fold_ema_f32(L.ptr(ws), b, c, k, L.ptr(hist), self._arr, self.rank, self.world, self.depth,
+                                                   int(slot), L.ptr(proto_old), ops.f32(eps), omd, d, L.ptr(new), L.ptr(sums),
+                                                   L.ptr(counts), L.ptr(hist_out), L.stream_of(ws)))
+        return new, sums, counts, hist_out
+
+    def _fold_outputs(self, proto_old, decay, out, want_sums, want_hist):
+        """Arguments and outputs of a fold launch: (proto_old, proto_new, 1 - decay, decay, sums, counts, hist), each output
+        None unless asked for (proto_new with ``decay``; it is ``out`` when given)."""
         dev = self.device
-        new = sums = counts = hist_out = None
+        new = sums = counts = hist = None
         omd = d = 0.0
         if decay is not None:
             proto_old = L.f32c(proto_old.detach())
@@ -191,12 +190,8 @@ class PeerExchange:
             sums = torch.empty((self.c, self.k), dtype=torch.float32, device=dev)
             counts = torch.empty((self.c,), dtype=torch.int64, device=dev)
         if want_hist:
-            hist_out = torch.empty((self.c + 1,), dtype=torch.int64, device=dev)
-        lib = L.bind(ws)
-        L.check(lib.uem_xchg_exchange_fold_ema_f32(L.ptr(ws), b, c, k, L.ptr(hist), self._arr, self.rank, self.world, self.depth,
-                                                   int(slot), L.ptr(proto_old), ops.f32(eps), omd, d, L.ptr(new), L.ptr(sums),
-                                                   L.ptr(counts), L.ptr(hist_out), L.stream_of(ws)))
-        return new, sums, counts, hist_out
+            hist = torch.empty((self.c + 1,), dtype=torch.int64, device=dev)
+        return proto_old, new, omd, d, sums, counts, hist
 
     def status(self):
         """Synchronises the current stream; 0 = fine, bit 8 = a bounded poll timed out (2 s)."""
