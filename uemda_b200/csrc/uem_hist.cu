@@ -66,24 +66,19 @@ __global__ void __launch_bounds__(kThreads) class_weight_lookup_kernel(const int
     }
 }
 
-// torch.histc (CPU) semantics: linear interpolation to a bin, then a local search against the
-// linspace bin edges; x outside [lo,hi] (or NaN) is dropped; x == hi lands in the last bin.
-__device__ __forceinline__ float hist_edge(int i, int bins, float lo, float hi, float step) {
-    return (i < (bins + 1) / 2) ? lo + step * (float)i : hi - step * (float)(bins - i);
-}
+// torch.histc semantics: bin = (int)((x - lo) * bins / (hi - lo)), each operation rounded in fp32 in that order, with no
+// search against the bin edges (a value on a computed edge may land one bin below it); x == hi lands in the last bin,
+// x outside [lo,hi] (or NaN) is dropped.
 __global__ void __launch_bounds__(kThreads) hist_f32_kernel(const float* __restrict__ x, int64_t n, int bins, float lo, float hi,
                                                             unsigned long long* __restrict__ hist) {
     extern __shared__ unsigned sh[];
     for (int i = threadIdx.x; i < bins; i += kThreads) sh[i] = 0;
     __syncthreads();
-    const float step = (hi - lo) / (float)bins;
+    const float range = __fsub_rn(hi, lo);
     for (int64_t i = (int64_t)blockIdx.x * kThreads + threadIdx.x; i < n; i += (int64_t)gridDim.x * kThreads) {
         const float v = x[i];
         if (!(v >= lo && v <= hi)) continue;
-        int pos = (int)((v - lo) / (hi - lo) * (float)bins);
-        pos = min(max(pos, 0), bins - 1);
-        if (pos > 0 && v < hist_edge(pos, bins, lo, hi, step)) --pos;
-        else if (pos < bins - 1 && v >= hist_edge(pos + 1, bins, lo, hi, step)) ++pos;
+        const int pos = min((int)__fdiv_rn(__fmul_rn(__fsub_rn(v, lo), (float)bins), range), bins - 1);
         atomicAdd(&sh[pos], 1u);
     }
     __syncthreads();

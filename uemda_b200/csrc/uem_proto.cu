@@ -501,7 +501,8 @@ extern "C" int uem_proto_accum_nchw_f32(const float* feat, int b, int k, int64_t
     cudaStream_t st = (cudaStream_t)stream;
     float* partial = (float*)ws;
     int* cnt_partial = (int*)proto_partials(ws, b, c, k).counts;
-    const bool vec = (hw % 4 == 0) && uem_aligned16(feat);
+    // the TMA form reads the labels in 16-byte loads (load_ids<4>): both maps must be 16-byte aligned
+    const bool vec = (hw % 4 == 0) && uem_aligned16(feat) && uem_aligned16(label);
     UEM_DISPATCH_C(c, {
         if (vec) {   // TMA form (hw fits int: at most 200K pixels)
             using P = ProtoTma<C, UEM_PROTO_RW>;
