@@ -376,6 +376,19 @@ UEM_API int uem_uvem_loss_backward_f32(const float* x1, const float* x2, int b, 
                                const int64_t* target, const float* coef, const float* scale, float* g1, float* g2,
                                void* ws, void* stream);
 
+/* ---- resident target set: a training batch cut from tile stores in HBM (SURVEY 8f-1; csrc/uem_store.cu) ----------------
+ * The loader's crop / flip / rot90 of the soft labels and superpixel map (augmentation.py:150-157, basedata.py:77-79,87) on
+ * the device.  soft_store (num_tiles,c,Hs,Ws) fp32, id_store (num_tiles,Hs,Ws) int32 (either may be NULL: its output is not
+ * written).  Sample s takes tile tiles[s] and windows[3s..3s+2] = (y0, x0, code), code = (t << 2) | (fy << 1) | fx:
+ *   win = store[tile, :, y0:y0+Hw, x0:x0+Ww], (Hw,Ww) = (Wo,Ho) if t else (Ho,Wo);
+ *   out[s] = win flipped on dim -2 if fy and on dim -1 if fx, then the last two dims transposed if t.
+ * soft_out (n,c,Ho,Wo) fp32, id_out (n,1,Ho,Wo) int64 (the ids widened exactly); a bit-exact permutation copy.
+ * A sample whose tile is outside [0,num_tiles), whose window leaves the tile or whose code is outside [0,8) reads nothing,
+ * gets zero outputs and sets bit 0 of *status (device int32, never cleared by the call).  One launch; n <= 65535. */
+UEM_API int uem_tile_gather(const float* soft_store, const int32_t* id_store, int64_t num_tiles, int c, int Hs, int Ws,
+                    const int64_t* tiles, const int32_t* windows /* (n,3): y0, x0, code */, int n, int Ho, int Wo,
+                    float* soft_out /* (n,c,Ho,Wo) */, int64_t* id_out /* (n,1,Ho,Wo) */, int32_t* status, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

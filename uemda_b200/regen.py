@@ -94,12 +94,14 @@ class PseudoLabelRegenerator:
         return ops.label_plus1_u8(self._chain(soft, sup, feat, preds))
 
     # ------------------------------------------------------------------ a whole (sharded) tile list
-    def run(self, batches, sink, rank=0, world_size=1, device=None):
-        """batches: a sequence of dicts {'soft', 'sup', 'feat', 'preds', 'names'} of HOST (ideally pinned) or device
-        tensors; this rank processes the contiguous slice mining.shard_range(len(batches), rank, world_size).
+    def run(self, batches, sink, rank=0, world_size=1, device=None, store=None):
+        """batches: a sequence of dicts {'soft', 'sup', 'feat', 'preds', 'names'[, 'tiles']} of HOST (ideally pinned) or
+        device tensors; this rank processes the contiguous slice mining.shard_range(len(batches), rank, world_size).
         sink(names, uint8 ndarray (b,H,W)) is called once per finished batch; the array lives in one of two reused pinned
         buffers and is only valid during the call (copy what must be kept).  Input staging and the copy back are
-        double-buffered.  Returns the number of tiles processed by this rank."""
+        double-buffered.  store: a store.TileStore; every staged batch's soft labels (and superpixel maps) are then also
+        written into it at the batch's 'tiles' indices, so the pass leaves the target set resident for self-training.
+        Returns the number of tiles processed by this rank."""
         device = device or torch.device("cuda", torch.cuda.current_device())
         lo, hi = mining.shard_range(len(batches), rank, world_size)
         copy_stream = torch.cuda.Stream(device=device)
@@ -134,6 +136,9 @@ class PseudoLabelRegenerator:
                     bt = batches[i]
                     nxt = {k: to_dev(bt.get(k)) for k in ("soft", "sup", "feat", "preds")}
                     nxt["names"] = bt.get("names")
+                    nxt["tiles"] = bt.get("tiles")
+                    if store is not None and nxt["tiles"] is None:
+                        raise ValueError("run(store=...): every batch needs its 'tiles' indices")
                     ev = torch.cuda.Event()
                     ev.record(copy_stream)
                     nxt["ready"] = ev
@@ -141,6 +146,8 @@ class PseudoLabelRegenerator:
                 cur.wait_event(staged["ready"])
                 for k in ("soft", "sup", "feat", "preds"):
                     hand_over(staged[k])
+                if store is not None:
+                    store.put(staged["tiles"], staged["soft"], staged["sup"])
                 u8 = self.process(staged["soft"], staged["sup"], staged["feat"], staged["preds"])
                 j = (i - 1 - lo) % 2
                 if host_bufs[j] is None or host_bufs[j].shape != u8.shape:
