@@ -389,6 +389,28 @@ UEM_API int uem_tile_gather(const float* soft_store, const int32_t* id_store, in
                     const int64_t* tiles, const int32_t* windows /* (n,3): y0, x0, code */, int n, int Ho, int Wo,
                     float* soft_out /* (n,c,Ho,Wo) */, int64_t* id_out /* (n,1,Ho,Wo) */, int32_t* status, void* stream);
 
+/* ---- resident source set: a source batch's labels and their DownscaleLabel cells cut from a uint8 store in HBM ----------
+ * The loader's decode, crop / flip / rot90 and int64 copy of the source label (train_ssl_uem.py:205,216,
+ * train_align_uem.py:147,150) and the DownscaleLabel of update_prototype / update_avg (alignment.py:86-90,484-509) on the
+ * device.  raw_store (num_tiles,Hs,Ws) uint8 holds the label files' bytes; lut (256) int64 maps a byte to its label.  Windows
+ * and codes as in uem_tile_gather:
+ *   label_out[s] = lut[D4(raw_store[tiles[s], y0:y0+Hw, x0:x0+Ww], code)]                  (n,Ho,Wo) int64, or NULL;
+ *   down_out[s]  = uem_downscale_label_i64(label_out[s], scale, n_classes, ignore_label, min_ratio)
+ *                                                                     (n,1,Ho/scale,Wo/scale) int64, or NULL.
+ * At least one output is given; down_out needs scale > 1 and n_classes in [1,UEM_MAX_CLASSES].  A power-of-two scale <= 16
+ * is counted in the gather's own launch (label_out may then be NULL); any other scale down-scales label_out (required) with
+ * uem_downscale_label_i64 in a second launch.  *status (device int32, never cleared by the call):
+ *   bit 0: a sample names a tile outside [0,num_tiles), a window outside the tile or a code outside [0,8); its label is
+ *          zero and its cells are those of a zero map (zero unless min_ratio > 1);
+ *   bit 1: down_out is given and a label of a window is outside {ignore_label} U [0,n_classes) (the reference's F.one_hot
+ *          over the whole label raises); such labels are not counted.
+ * n <= 65535. */
+UEM_API int uem_label_gather_u8(const uint8_t* raw_store, int64_t num_tiles, int Hs, int Ws, const int64_t* lut /* 256 */,
+                        const int64_t* tiles, const int32_t* windows /* (n,3) */, int n, int Ho, int Wo,
+                        int64_t* label_out /* (n,Ho,Wo) or NULL */, int scale, int n_classes, int64_t ignore_label,
+                        float min_ratio, int64_t* down_out /* (n,1,Ho/scale,Wo/scale) or NULL */, int32_t* status,
+                        void* stream);
+
 #ifdef __cplusplus
 }
 #endif

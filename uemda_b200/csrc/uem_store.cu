@@ -8,6 +8,10 @@
 // backwards), so each warp loads and stores 32 consecutive words directly.  Transposing codes map an output row to a
 // source column: the CTA loads the TX x TY source block of every plane row by row into shared memory (cp.async, one
 // stage per plane, one barrier) and stores it column by column, so both sides stay coalesced.  Loads are 4-byte, so an arbitrary (unaligned) window offset costs nothing extra.
+//
+// Resident source set: each source batch's labels cut from the label files' own bytes kept in HBM, together with the
+// DownscaleLabel cells that update_prototype / update_avg take (train_ssl_uem.py:205,216, train_align_uem.py:147,150,
+// alignment.py:86-90,484-509): label_gather_kernel below.
 #include "uem_common.cuh"
 #include "uem_tma.cuh"  // smem_u32
 
@@ -144,6 +148,145 @@ __global__ void __launch_bounds__(kThreads, 6) tile_gather_kernel(const float* _
     if (id_store) store_plane<int32_t, int64_t>(stage + cs * kStage, iout, g);
 }
 
+// ------------------------------------------------------------------------------- resident source set
+// Label maps stored as the label files' bytes, mapped through a 256-entry LUT.  Every code goes through one byte stage
+// in output order (transposing codes load it column-wise like stage_plane), so loads and int64 stores stay coalesced and
+// the cell counts read the same stage.  With a power-of-two scale <= TY, the 16-row CTA tile holds whole cells: 4 pixels
+// per thread, the s*s/4 threads of a cell consecutive, their packed counts folded by xor-shuffles within a warp and by
+// shared memory across the two warps of a 16 x 16 cell.  A cell has at most 256 pixels, so a count fits 9 bits: classes
+// 0-6 are fields of a 64-bit word, class 7 and the ignore bin fields of a 32-bit word, and a pixel adds its byte's
+// increments from shared memory (no branch on the class).
+constexpr int kLabPitch = TX + 4;             // bytes per stage row
+constexpr uint32_t kIncBad = 1u << 31;        // in inc_hi: the label is outside {ignore} U [0,n_classes) (not counted; bit 31 of
+                                              // a sum is never read)
+
+struct LabelSmem {
+    int64_t lut[256];
+    uint64_t inc_lo[256];                     // byte -> 1 << 9c for class c < 7
+    uint32_t inc_hi[256];                     // byte -> 1 for class 7, 1 << 9 for the ignore label, kIncBad
+    uint8_t stage[TY * kLabPitch];            // [row][col] of the CTA's output tile, as stored bytes
+    uint64_t lo[kThreads];                    // per lane group: the summed increments
+    uint32_t hi[kThreads];
+};
+
+// count of bin ci (0..7 = classes, 8 = ignore)
+__device__ __forceinline__ unsigned bin_count(uint64_t lo, uint32_t hi, int ci) {
+    return ci < 7 ? (unsigned)(lo >> (9 * ci)) & 0x1ffu : (hi >> (9 * (ci - 7))) & 0x1ffu;
+}
+
+// check: flag labels outside {ignore} U [0,n_classes) in bit 1 of status.  S: 0, or the power of two <= TY whose cells are
+// counted here into down_out (n,1,Ho/S,Wo/S).  An invalid sample writes a zero label and the cells of a zero map.
+template <int S>
+__global__ void __launch_bounds__(kThreads) label_gather_kernel(const uint8_t* __restrict__ raw, int64_t num_tiles, int Hs, int Ws,
+                                                                const int64_t* __restrict__ lut, const int64_t* __restrict__ tiles,
+                                                                const int32_t* __restrict__ windows, int Ho, int Wo,
+                                                                int64_t* __restrict__ label_out, int check, int n_classes,
+                                                                int64_t ignore_label, float min_ratio, int64_t* __restrict__ down_out,
+                                                                int32_t* __restrict__ status) {
+    static_assert(kThreads == 256, "one thread per LUT entry");
+    static_assert(S == 0 || (S >= 2 && S <= TY && (S & (S - 1)) == 0 && TX % S == 0), "cells must lie inside the CTA tile");
+    __shared__ LabelSmem sm;
+    const int n = blockIdx.z, oy0 = blockIdx.y * TY, ox0 = blockIdx.x * TX;
+    const Sample s = read_sample(tiles, windows, n, num_tiles, Hs, Ws, Ho, Wo);
+    if (!s.ok && blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) atomicOr(status, 1);
+    {
+        const int64_t v = lut[threadIdx.x];
+        const bool ign = v == ignore_label, cls = !ign && v >= 0 && v < n_classes;
+        sm.lut[threadIdx.x] = v;
+        sm.inc_lo[threadIdx.x] = cls && v < 7 ? 1ull << (9 * v) : 0ull;
+        sm.inc_hi[threadIdx.x] = ign ? 1u << 9 : (cls ? (v == 7 ? 1u : 0u) : kIncBad);
+    }
+    if (s.ok) {
+        const uint8_t* in = raw + s.tile * ((int64_t)Hs * Ws) + s.src;
+        if (!s.t) {  // out[oy, ox] = win[fy ? Ho-1-oy : oy, fx ? Wo-1-ox : ox]
+            const int ty = threadIdx.x / TX, tx = threadIdx.x % TX, ox = ox0 + tx, oy = oy0 + ty;
+            if (ox < Wo) {
+                const uint8_t* p = in + (int64_t)(s.fy ? Ho - 1 - oy : oy) * Ws + (s.fx ? Wo - 1 - ox : ox);
+                const int64_t step = s.fy ? -(int64_t)kRows * Ws : (int64_t)kRows * Ws;
+#pragma unroll
+                for (int i = 0; i < kPer; ++i)
+                    if (oy + i * kRows < Ho) sm.stage[(ty + i * kRows) * kLabPitch + tx] = __ldcs(p + i * step);
+            }
+        } else {     // out[oy, ox] = win[fy ? Wo-1-ox : ox, fx ? Ho-1-oy : oy]: a warp reads 16 bytes of 2 source rows
+            const int q = threadIdx.x % TY, c0 = threadIdx.x / TY, oy = oy0 + q, ox = ox0 + c0;
+            if (oy < Ho) {
+                const uint8_t* p = in + (int64_t)(s.fy ? Wo - 1 - ox : ox) * Ws + (s.fx ? Ho - 1 - oy : oy);
+                const int64_t step = s.fy ? -(int64_t)kCols * Ws : (int64_t)kCols * Ws;
+#pragma unroll
+                for (int i = 0; i < kPer; ++i)
+                    if (ox + i * kCols < Wo) sm.stage[q * kLabPitch + c0 + i * kCols] = __ldcs(p + i * step);
+            }
+        }
+    }
+    __syncthreads();
+    int bad = 0;
+    {   // labels, row-major: a warp stores 32 consecutive int64
+        const int ty = threadIdx.x / TX, tx = threadIdx.x % TX, ox = ox0 + tx;
+        if (ox < Wo) {
+            const int64_t o = ((int64_t)n * Ho + oy0 + ty) * Wo + ox;
+#pragma unroll
+            for (int i = 0; i < kPer; ++i) {
+                const int r = ty + i * kRows;
+                if (oy0 + r >= Ho) break;
+                int64_t v = 0;
+                if (s.ok) {
+                    const int b = sm.stage[r * kLabPitch + tx];
+                    v = sm.lut[b];
+                    bad |= sm.inc_hi[b] == kIncBad;
+                }
+                if (label_out) label_out[o + (int64_t)i * kRows * Wo] = v;
+            }
+        }
+    }
+    // cells, cell-major: thread t counts pixels 4(t % G) .. +3 (row-major within the cell) of cell t / G
+    constexpr int G = S * S / 4, kLanes = G < 32 ? G : 32, kCpr = S ? TX / S : 1;
+    if (S) {
+        const int cell = threadIdx.x / G, k0 = (threadIdx.x % G) * 4;
+        const uint8_t* st = sm.stage + (cell / kCpr * S) * kLabPitch + cell % kCpr * S;
+        uint64_t lo = 0ull;
+        uint32_t hi = 0u;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const int k = k0 + j;
+            // an invalid sample counts its zero map (byte 0 stands in; sm.lut[0] is not used); pixels past the output edge
+            // belong to cells that are not written
+            const int b = s.ok ? st[(k / S) * kLabPitch + k % S] : 0;
+            lo += s.ok ? sm.inc_lo[b] : (ignore_label == 0 ? 0ull : 1ull);
+            hi += s.ok ? sm.inc_hi[b] : (ignore_label == 0 ? 1u << 9 : 0u);
+        }
+#pragma unroll
+        for (int o = kLanes >> 1; o > 0; o >>= 1) {
+            lo += __shfl_xor_sync(0xffffffffu, lo, o);
+            hi += __shfl_xor_sync(0xffffffffu, hi, o);
+        }
+        if (threadIdx.x % kLanes == 0) {
+            sm.lo[threadIdx.x / kLanes] = lo;
+            sm.hi[threadIdx.x / kLanes] = hi;
+        }
+    }
+    if (__syncthreads_or(bad) && check && threadIdx.x == 0) atomicOr(status, 2);
+    if (!S) return;
+    constexpr int kPerCell = S ? G / kLanes : 1;
+    const int h = Ho / S, w = Wo / S;
+    const int cell = threadIdx.x, cy = oy0 / S + cell / kCpr, cx = ox0 / S + cell % kCpr;
+    if (cell >= (S ? TY * TX / (S * S) : 0) || cy >= h || cx >= w) return;
+    uint64_t lo = sm.lo[cell * kPerCell];
+    uint32_t hi = sm.hi[cell * kPerCell];
+#pragma unroll
+    for (int g = 1; g < kPerCell; ++g) {
+        lo += sm.lo[cell * kPerCell + g];
+        hi += sm.hi[cell * kPerCell + g];
+    }
+    unsigned best = bin_count(lo, hi, 0);
+    int arg = 0;
+#pragma unroll
+    for (int ci = 1; ci < 8; ++ci)
+        if (ci < n_classes && bin_count(lo, hi, ci) > best) { best = bin_count(lo, hi, ci); arg = ci; }  // first index wins ties
+    if (bin_count(lo, hi, 8) > best) { best = bin_count(lo, hi, 8); arg = 8; }   // the ignore bin is last (alignment.py:497)
+    const float ratio = __fdiv_rn((float)best, (float)(S * S));   // avg_pool2d of the one-hot: count / (s*s)
+    down_out[((int64_t)n * h + cy) * w + cx] = (arg == 8 || ratio < min_ratio) ? ignore_label : (int64_t)arg;
+}
+
 }  // namespace
 
 extern "C" int uem_tile_gather(const float* soft_store, const int32_t* id_store, int64_t num_tiles, int c, int Hs, int Ws,
@@ -164,4 +307,40 @@ extern "C" int uem_tile_gather(const float* soft_store, const int32_t* id_store,
                                                                     soft_out, id_out, status);
     UEM_CHECK_LAUNCH();
     return 0;
+}
+
+extern "C" int uem_label_gather_u8(const uint8_t* raw_store, int64_t num_tiles, int Hs, int Ws, const int64_t* lut,
+                                   const int64_t* tiles, const int32_t* windows, int n, int Ho, int Wo, int64_t* label_out,
+                                   int scale, int n_classes, int64_t ignore_label, float min_ratio, int64_t* down_out,
+                                   int32_t* status, void* stream) {
+    UEM_REQUIRE((raw_store || num_tiles == 0) && lut && tiles && windows && status && n >= 0 && n <= 65535 && num_tiles >= 0 &&
+                    Hs > 0 && Ws > 0 && Ho > 0 && Wo > 0,
+                "uem_label_gather_u8: bad arguments");
+    UEM_REQUIRE(label_out || down_out, "uem_label_gather_u8: no output (label_out and down_out are both NULL)");
+    UEM_REQUIRE(!down_out || (scale > 1 && n_classes >= 1 && n_classes <= UEM_MAX_C),
+                "uem_label_gather_u8: down_out needs scale > 1 (got %d) and n_classes in [1,%d] (got %d)", scale, UEM_MAX_C, n_classes);
+    // a power-of-two scale <= TY: every cell lies inside one CTA tile and is counted there; any other scale down-scales the
+    // written labels with uem_downscale_label_i64 in a second launch
+    const bool fused = down_out && scale <= TY && (scale & (scale - 1)) == 0;
+    UEM_REQUIRE(!down_out || fused || label_out, "uem_label_gather_u8: scale %d is down-scaled from label_out, which is NULL", scale);
+    if (n == 0) return 0;
+    const dim3 grid(uem_div_up(Wo, TX), uem_div_up(Ho, TY), n);
+    UEM_REQUIRE(grid.y <= 65535, "uem_label_gather_u8: output height %d too large", Ho);
+    const cudaStream_t st = (cudaStream_t)stream;
+    const int check = down_out ? 1 : 0;
+#define UEM_LABEL_GATHER(S_)                                                                                                     \
+    label_gather_kernel<S_><<<grid, kThreads, 0, st>>>(raw_store, num_tiles, Hs, Ws, lut, tiles, windows, Ho, Wo, label_out, check, \
+                                                       n_classes, ignore_label, min_ratio, down_out, status)
+    switch (fused ? scale : 0) {
+        case 2: UEM_LABEL_GATHER(2); break;
+        case 4: UEM_LABEL_GATHER(4); break;
+        case 8: UEM_LABEL_GATHER(8); break;
+        case 16: UEM_LABEL_GATHER(16); break;
+        default: UEM_LABEL_GATHER(0); break;
+    }
+#undef UEM_LABEL_GATHER
+    UEM_CHECK_LAUNCH();
+    if (!down_out || fused) return 0;
+    // bit 1 is already set from every label of the window; the down-scale's own check would report the same labels as bit 0
+    return uem_downscale_label_i64(label_out, n, Ho, Wo, scale, n_classes, ignore_label, min_ratio, down_out, nullptr, stream);
 }

@@ -6,15 +6,68 @@ during self-training the loader reads them back with the int32 superpixel .tif (
 crop / flip / rot90 to both (augmentation.py:150-157) and the step copies them to the device (train_ssl_uem.py:199-201).
 Here the loader returns ``(index, y0, x0, code)`` per sample and ``TileStore.batch`` produces ``label_t_soft`` (n,c,Ho,Wo)
 fp32 and ``label_t_sup`` (n,1,Ho,Wo) int64 in one launch (uem_tile_gather): only the augmentation parameters cross PCIe.
+
+Resident source set: the source label files' bytes kept in HBM.  The loader decodes the label PNG, crops / flips / rotates it,
+widens it to int64 (train_ssl_uem.py:205,216, train_align_uem.py:147,150) and the step down-scales it again for the
+prototypes (alignment.py:86-90,484-509).  ``LabelStore.batch`` produces ``label_s`` and its DownscaleLabel cells in one
+launch (uem_label_gather_u8) from the same ``(index, y0, x0, code)`` per sample.
 """
 import torch
 
 from . import _lib as L
 from . import config
+from .ops import f32
 
-__all__ = ["TileStore"]
+__all__ = ["TileStore", "LabelStore"]
 
 _I32_MIN, _I32_MAX = -2 ** 31, 2 ** 31 - 1
+
+
+def _cuda_device(device, what):
+    device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+    if device.type != "cuda":
+        raise L.UemLibraryError("%s lives on a CUDA device (got %s)" % (what, device))
+    return device
+
+
+def _tile_list(tiles, b, num_tiles):
+    tiles = [int(t) for t in (tiles.tolist() if torch.is_tensor(tiles) else tiles)]
+    if len(tiles) != b:
+        raise ValueError("put: %d tile indices for a batch of %d" % (len(tiles), b))
+    bad = [t for t in tiles if not 0 <= t < num_tiles]
+    if bad:
+        raise IndexError("put: tile index %d outside [0, %d)" % (bad[0], num_tiles))
+    return tiles
+
+
+def _runs(tiles):
+    """(first tile, i, j) per run tiles[i:j] of consecutive tile indices: one copy each."""
+    i, b = 0, len(tiles)
+    while i < b:
+        j = i + 1
+        while j < b and tiles[j] == tiles[j - 1] + 1:
+            j += 1
+        yield tiles[i], i, j
+        i = j
+
+
+def _stage(tiles, windows, dev):
+    """Host index lists -> device tensors with one small copy; device tensors pass through (graph-capturable)."""
+    if torch.is_tensor(tiles) and tiles.is_cuda and torch.is_tensor(windows) and windows.is_cuda:
+        return (tiles.to(device=dev, dtype=torch.int64).contiguous().view(-1),
+                windows.to(device=dev, dtype=torch.int32).contiguous().view(-1, 3))
+    t = torch.as_tensor(tiles.cpu() if torch.is_tensor(tiles) else tiles, dtype=torch.int64).reshape(-1)
+    w = torch.as_tensor(windows.cpu() if torch.is_tensor(windows) else windows, dtype=torch.int32).reshape(-1, 3)
+    n = t.numel()
+    host = torch.empty(5 * n, dtype=torch.int32, pin_memory=True)   # [n int64 tiles | n x 3 int32 windows]
+    host[:2 * n].view(torch.int64).copy_(t)
+    host[2 * n:].copy_(w.reshape(-1))
+    staged = host.to(dev, non_blocking=True)
+    return staged[:2 * n].view(torch.int64), staged[2 * n:].view(-1, 3)
+
+
+def _size(size):
+    return (int(size), int(size)) if isinstance(size, int) else (int(size[0]), int(size[1]))
 
 
 class TileStore:
@@ -22,9 +75,7 @@ class TileStore:
     allocation, zero until ``put``.  ``superpixels=False`` keeps soft labels only (``ids`` is None)."""
 
     def __init__(self, num_tiles, class_num, height, width, device=None, superpixels=True):
-        device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
-        if device.type != "cuda":
-            raise L.UemLibraryError("TileStore lives on a CUDA device (got %s)" % device)
+        device = _cuda_device(device, "TileStore")
         self.shape = (int(num_tiles), int(class_num), int(height), int(width))
         self.soft = torch.zeros(self.shape, dtype=torch.float32, device=device)
         self.ids = torch.zeros((self.shape[0],) + self.shape[2:], dtype=torch.int32, device=device) if superpixels else None
@@ -47,15 +98,6 @@ class TileStore:
         if k in (2, 3):
             fy ^= 1
         return ((k & 1) << 2) | (fy << 1) | fx
-
-    def _tile_list(self, tiles, b):
-        tiles = [int(t) for t in (tiles.tolist() if torch.is_tensor(tiles) else tiles)]
-        if len(tiles) != b:
-            raise ValueError("put: %d tile indices for a batch of %d" % (len(tiles), b))
-        bad = [t for t in tiles if not 0 <= t < self.shape[0]]
-        if bad:
-            raise IndexError("put: tile index %d outside [0, %d)" % (bad[0], self.shape[0]))
-        return tiles
 
     def put(self, tiles, soft, sup=None):
         """Writes soft (b,c,H,W) and, if given, sup ((b,1,H,W) or (b,H,W), int64 or int32) at the tile indices ``tiles``
@@ -80,33 +122,10 @@ class TileStore:
                 lo, hi = int(sup.min()), int(sup.max())
                 if lo < _I32_MIN or hi > _I32_MAX:
                     raise RuntimeError("put: superpixel id %d outside the int32 range of the store" % (lo if lo < _I32_MIN else hi))
-        tiles = self._tile_list(tiles, b)
-        # one copy per run of consecutive tile indices
-        i = 0
-        while i < b:
-            j = i + 1
-            while j < b and tiles[j] == tiles[j - 1] + 1:
-                j += 1
-            t = tiles[i]
+        for t, i, j in _runs(_tile_list(tiles, b, self.shape[0])):
             self.soft[t:t + j - i].copy_(soft[i:j], non_blocking=True)
             if sup is not None:
                 self.ids[t:t + j - i].copy_(sup[i:j], non_blocking=True)
-            i = j
-
-    def _stage(self, tiles, windows):
-        """Host index lists -> device tensors with one small copy; device tensors pass through (graph-capturable)."""
-        dev = self.device
-        if torch.is_tensor(tiles) and tiles.is_cuda and torch.is_tensor(windows) and windows.is_cuda:
-            return (tiles.to(device=dev, dtype=torch.int64).contiguous().view(-1),
-                    windows.to(device=dev, dtype=torch.int32).contiguous().view(-1, 3))
-        t = torch.as_tensor(tiles.cpu() if torch.is_tensor(tiles) else tiles, dtype=torch.int64).reshape(-1)
-        w = torch.as_tensor(windows.cpu() if torch.is_tensor(windows) else windows, dtype=torch.int32).reshape(-1, 3)
-        n = t.numel()
-        host = torch.empty(5 * n, dtype=torch.int32, pin_memory=True)   # [n int64 tiles | n x 3 int32 windows]
-        host[:2 * n].view(torch.int64).copy_(t)
-        host[2 * n:].copy_(w.reshape(-1))
-        staged = host.to(dev, non_blocking=True)
-        return staged[:2 * n].view(torch.int64), staged[2 * n:].view(-1, 3)
 
     def batch(self, tiles, windows, size, out=None):
         """Cuts one batch: sample s is ``store[tiles[s]]`` at window (y0, x0) = windows[s][:2] under code windows[s][2]
@@ -115,8 +134,8 @@ class TileStore:
         and ``out`` make the call capturable in a CUDA graph (with config.strict_asserts off); host sequences are staged
         with one small copy.  Under config.strict_asserts an out-of-range sample raises (one read-back of the status word,
         which is then cleared); otherwise its outputs are zero and ``status`` keeps bit 0 set."""
-        Ho, Wo = (int(size), int(size)) if isinstance(size, int) else (int(size[0]), int(size[1]))
-        tiles, windows = self._stage(tiles, windows)
+        Ho, Wo = _size(size)
+        tiles, windows = _stage(tiles, windows, self.device)
         n = tiles.numel()
         if windows.shape[0] != n:
             raise ValueError("batch: %d tile indices but %d windows" % (n, windows.shape[0]))
@@ -144,3 +163,88 @@ class TileStore:
                 raise IndexError("TileStore.batch: a sample names a tile outside [0, %d) or a window outside the %dx%d tile"
                                  % (T, H, W))
         return soft, sup
+
+
+class LabelStore:
+    """``raw``: (T,H,W) uint8, the source label files' own bytes, one allocation, zero until ``put``.  ``lut``: 256 int64
+    on the device, the loader's byte -> label mapping (LoveDA: ``0 -> -1, v -> v - 1``; an ignore byte: ``255 -> -1``),
+    validated here.  ``batch`` cuts a batch with the windows and codes of ``TileStore.batch`` (``TileStore.d4_code``)."""
+
+    def __init__(self, num_tiles, height, width, lut, device=None):
+        lut = torch.as_tensor(lut)
+        if lut.dim() != 1 or lut.numel() != 256:
+            raise ValueError("LabelStore: lut must map each of the 256 byte values (got shape %s)" % (tuple(lut.shape),))
+        if lut.is_floating_point() or lut.is_complex() or lut.dtype == torch.bool:
+            raise TypeError("LabelStore: lut must hold integer labels (got %s)" % lut.dtype)
+        device = _cuda_device(device, "LabelStore")
+        self.shape = (int(num_tiles), int(height), int(width))
+        self.raw = torch.zeros(self.shape, dtype=torch.uint8, device=device)
+        self.lut = lut.to(device=device, dtype=torch.int64).contiguous()
+        # bit 0: a sample of a batch() named a tile outside the store or a window outside the tile;
+        # bit 1: a batch() with downscale met a label outside {ignore} U [0, n_classes)
+        self.status = torch.zeros(1, dtype=torch.int32, device=device)
+
+    @property
+    def device(self):
+        return self.raw.device
+
+    def put(self, tiles, raw):
+        """Writes raw (b,H,W) or (b,1,H,W) uint8 label bytes at the tile indices ``tiles`` (a sequence or a tensor of b
+        indices), from the host (pinned: the copies are asynchronous) or the device, on the current stream."""
+        if raw.dtype != torch.uint8:
+            raise TypeError("put: label bytes must be uint8 (got %s)" % raw.dtype)
+        if raw.dim() == 4:
+            if raw.shape[1] != 1:
+                raise ValueError("put: label maps must be (b,1,H,W) or (b,H,W)")
+            raw = raw[:, 0]
+        if raw.dim() != 3 or tuple(raw.shape[1:]) != self.shape[1:]:
+            raise ValueError("put: label maps of shape %s do not fit a store of %s" % (tuple(raw.shape), self.shape))
+        for t, i, j in _runs(_tile_list(tiles, raw.shape[0], self.shape[0])):
+            self.raw[t:t + j - i].copy_(raw[i:j], non_blocking=True)
+
+    def batch(self, tiles, windows, size, downscale=None, out=None):
+        """Cuts one batch: label[s] = lut[store[tiles[s]] at window (y0, x0) = windows[s][:2] under code windows[s][2]],
+        size = (Ho, Wo) or an int, and with ``downscale`` (a DownscaleLabel, e.g. ``aligner.downscale_gt``) its cells
+        down[s] = downscale(label[s]) in the same launch.  Returns (label (n,Ho,Wo) int64, down (n,1,Ho//s,Wo//s) int64 or
+        None), written into ``out`` = (label, down) when given.  tiles (n,) int64 / windows (n,3) int32 device tensors and
+        ``out`` make the call capturable in a CUDA graph (with config.strict_asserts off).  An out-of-range sample gets a
+        zero label (and the cells of a zero map) and sets bit 0 of ``status``; with ``downscale``, a label outside
+        {ignore} U [0, n_classes) sets bit 1 and is not counted.  Under config.strict_asserts the call reads the word back,
+        clears it and raises IndexError for bit 0, or DownscaleLabel's RuntimeError for bit 1."""
+        Ho, Wo = _size(size)
+        tiles, windows = _stage(tiles, windows, self.device)
+        n = tiles.numel()
+        if windows.shape[0] != n:
+            raise ValueError("batch: %d tile indices but %d windows" % (n, windows.shape[0]))
+        T, H, W = self.shape
+        scale = n_classes = ignore = 0
+        min_ratio = 0.0
+        if downscale is not None:
+            scale, n_classes = int(downscale.scale_factor), int(downscale.n_classes)
+            ignore, min_ratio = int(downscale.ignore_label), f32(downscale.min_ratio)
+        dshape = (n, 1, Ho // scale, Wo // scale) if downscale is not None else None
+        if out is None:
+            label = torch.empty((n, Ho, Wo), dtype=torch.int64, device=self.device)
+            down = torch.empty(dshape, dtype=torch.int64, device=self.device) if dshape else None
+        else:
+            label, down = out
+            for name, t, shape in (("label", label, (n, Ho, Wo)), ("down", down, dshape)):
+                if shape and (t is None or t.shape != shape or t.dtype != torch.int64 or t.device != self.device
+                              or not t.is_contiguous()):
+                    raise ValueError("batch: out %s must be a contiguous %s int64 tensor on %s" % (name, shape, self.device))
+            if dshape is None:
+                down = None
+        lib = L.bind(self.raw)
+        L.check(lib.uem_label_gather_u8(L.ptr(self.raw), T, H, W, L.ptr(self.lut), L.ptr(tiles), L.ptr(windows), n, Ho, Wo,
+                                        L.ptr(label), scale, n_classes, ignore, min_ratio, L.ptr(down), L.ptr(self.status),
+                                        L.stream_of(self.raw)))
+        if config.strict_asserts:
+            bits = int(self.status.item())
+            if bits:
+                self.status.zero_()
+                if bits & 1:
+                    raise IndexError("LabelStore.batch: a sample names a tile outside [0, %d) or a window outside the %dx%d "
+                                     "tile" % (T, H, W))
+                # F.one_hot in the reference (alignment.py:502) rejects these
+                raise RuntimeError("Class values must be non-negative and smaller than num_classes.")
+        return label, down
