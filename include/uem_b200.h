@@ -411,6 +411,19 @@ UEM_API int uem_label_gather_u8(const uint8_t* raw_store, int64_t num_tiles, int
                         float min_ratio, int64_t* down_out /* (n,1,Ho/scale,Wo/scale) or NULL */, int32_t* status,
                         void* stream);
 
+/* ---- resident image set: a batch's normalised images cut from a uint8 store in HBM ------------------------------------
+ * The loader's crop / flip / rot90 of the image (augmentation.py:150-157), its per-channel byte -> value map (e.g.
+ * albumentations' Normalize) and the batch's host -> device copy, on the device.  store (num_tiles,Hs,Ws,C) uint8,
+ * interleaved as decoded image files are, C in [1,4]; table (C,256) fp32 maps a byte of channel ch to its value.  Windows and codes as in uem_tile_gather:
+ *   out[s, ch] = table[ch][D4(store[tiles[s], y0:y0+Hw, x0:x0+Ww, ch], code)]                      (n,C,Ho,Wo) fp32;
+ * a flip reverses the pixel order of the window, never the channel order of a pixel.  16-byte stores when Wo % 4 == 0
+ * and out is 16-byte aligned, 4-byte stores otherwise.  A sample whose tile is outside [0,num_tiles), whose window leaves
+ * the tile or whose code is outside [0,8) reads nothing, gets zero planes and sets bit 0 of *status (device int32, never
+ * cleared by the call).  Byte offsets are 64-bit.  One launch; n <= 65535. */
+UEM_API int uem_image_gather_u8(const uint8_t* store, int64_t num_tiles, int Hs, int Ws, int C, const float* table /* C x 256 */,
+                        const int64_t* tiles, const int32_t* windows /* (n,3) */, int n, int Ho, int Wo,
+                        float* out /* (n,C,Ho,Wo) */, int32_t* status, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -98,6 +98,7 @@ SIGNATURES = {
     "uem_uvem_loss_backward_f32": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P]),
     "uem_tile_gather": (_I, [_P, _P, _L, _I, _I, _I, _P, _P, _I, _I, _I, _P, _P, _P, _P]),
     "uem_label_gather_u8": (_I, [_P, _L, _I, _I, _P, _P, _P, _I, _I, _I, _P, _I, _I, _L, _F, _P, _P, _P]),
+    "uem_image_gather_u8": (_I, [_P, _L, _I, _I, _I, _P, _P, _P, _I, _I, _I, _P, _P, _P]),
 }
 
 _lock = threading.Lock()

@@ -12,6 +12,10 @@
 // Resident source set: each source batch's labels cut from the label files' own bytes kept in HBM, together with the
 // DownscaleLabel cells that update_prototype / update_avg take (train_ssl_uem.py:205,216, train_align_uem.py:147,150,
 // alignment.py:86-90,484-509): label_gather_kernel below.
+//
+// Resident image set: each batch's images cut from the decoded image bytes kept in HBM and mapped through a per-channel
+// byte -> value table (the image's crop / flip / rot90 of augmentation.py:150-157 and its normalisation):
+// image_gather_kernel below.
 #include "uem_common.cuh"
 #include "uem_tma.cuh"  // smem_u32
 
@@ -287,6 +291,86 @@ __global__ void __launch_bounds__(kThreads) label_gather_kernel(const uint8_t* _
     down_out[((int64_t)n * h + cy) * w + cx] = (arg == 8 || ratio < min_ratio) ? ignore_label : (int64_t)arg;
 }
 
+// ------------------------------------------------------------------------------- resident image set
+// Images stored as decoded (T,Hs,Ws,C) uint8 (interleaved), each byte mapped through its channel's 256-entry fp32 table.
+// A segment is the run of pixels that is contiguous in the source for one CTA tile: an output row (TX pixels) without a
+// transpose, an output column (TY pixels) with one; its P * C bytes are read forwards whatever the flip, and a flip only
+// reverses the pixel order in which they are staged (the C bytes of a pixel keep their order).  Byte loads: any x0 works.
+template <int C>
+constexpr int kImgPitch = TX * C + 4;  // bytes per stage row: an odd number of words, so column-wise stage writes spread over banks
+
+template <int C>
+struct ImageSmem {
+    float table[C][256];
+    uint8_t stage[TY * kImgPitch<C>];  // [row q][column x][channel] of the CTA's output tile, as stored bytes
+};
+
+// segment k (k < nseg) starts at src + k * seg_step; its pixel p (p < npix) goes to output pixel flip ? npix-1-p : p of the
+// segment, staged at k * seg_pitch + pixel * pix_pitch
+template <int C, int P>
+__device__ __forceinline__ void stage_image(const uint8_t* __restrict__ src, int64_t seg_step, int nseg, int npix, bool flip,
+                                            uint8_t* stage, int seg_pitch, int pix_pitch) {
+    constexpr int kSeg = P * C;
+#pragma unroll
+    for (int i = 0; i < TY * TX * C / kThreads; ++i) {
+        const int l = threadIdx.x + i * kThreads, k = l / kSeg, j = l % kSeg, p = j / C;
+        if (k < nseg && p < npix)
+            stage[k * seg_pitch + (flip ? npix - 1 - p : p) * pix_pitch + j % C] = __ldcs(src + k * seg_step + j);
+    }
+}
+
+// VW = 4: 16-byte stores (Wo % 4 == 0 and out 16-byte aligned); VW = 1: 4-byte stores.  An invalid sample writes zeros.
+template <int C, int VW>
+__global__ void __launch_bounds__(kThreads) image_gather_kernel(const uint8_t* __restrict__ raw, int64_t num_tiles, int Hs, int Ws,
+                                                                const float* __restrict__ table, const int64_t* __restrict__ tiles,
+                                                                const int32_t* __restrict__ windows, int Ho, int Wo,
+                                                                float* __restrict__ out, int32_t* __restrict__ status) {
+    static_assert(C >= 1 && C <= 4 && (VW == 1 || VW == 4), "1 to 4 channels; 4-byte or 16-byte stores");
+    __shared__ ImageSmem<C> sm;
+    const int n = blockIdx.z;
+    const Geo g{Ws, Ho, Wo, (int)blockIdx.y * TY, (int)blockIdx.x * TX};
+    const Sample s = read_sample(tiles, windows, n, num_tiles, Hs, Ws, Ho, Wo);
+    if (!s.ok && blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) atomicOr(status, 1);
+#pragma unroll
+    for (int ch = 0; ch < C; ++ch) sm.table[ch][threadIdx.x] = table[ch * 256 + threadIdx.x];
+    const int rows = min(TY, Ho - g.oy0), cols = min(TX, Wo - g.ox0);
+    if (s.ok) {
+        const uint8_t* in = raw + (s.tile * Hs * Ws + s.src) * C;
+        const int64_t row = (int64_t)Ws * C;
+        if (!s.t) {  // segment q = output row oy0 + q: window row fy ? Ho-1-oy : oy, columns of ox0 .. ox0+cols-1
+            const int wy = s.fy ? Ho - 1 - g.oy0 : g.oy0, wx = s.fx ? Wo - g.ox0 - cols : g.ox0;
+            stage_image<C, TX>(in + wy * row + wx * C, s.fy ? -row : row, rows, cols, s.fx, sm.stage, kImgPitch<C>, C);
+        } else {     // segment r = output column ox0 + r: window row fy ? Wo-1-ox : ox, columns of oy0 .. oy0+rows-1
+            const int wy = s.fy ? Wo - 1 - g.ox0 : g.ox0, wx = s.fx ? Ho - g.oy0 - rows : g.oy0;
+            stage_image<C, TY>(in + wy * row + wx * C, s.fy ? -row : row, cols, rows, s.fx, sm.stage, C, kImgPitch<C>);
+        }
+    }
+    __syncthreads();
+    // row-major stores: a warp writes 32 x VW consecutive floats of one plane
+    constexpr int kLanes = TX / VW, kStep = kThreads / kLanes;
+    const int x = threadIdx.x % kLanes * VW, q0 = threadIdx.x / kLanes;
+    if (x >= cols) return;
+    const int64_t plane = (int64_t)Ho * Wo;
+    float* o = out + (int64_t)n * C * plane + (int64_t)(g.oy0 + q0) * Wo + g.ox0 + x;
+#pragma unroll
+    for (int i = 0; i < TY / kStep; ++i) {
+        const int q = q0 + i * kStep;
+        if (q >= rows) break;
+        const uint8_t* px = sm.stage + q * kImgPitch<C> + x * C;
+#pragma unroll
+        for (int ch = 0; ch < C; ++ch) {
+            float v[VW];
+#pragma unroll
+            for (int k = 0; k < VW; ++k) v[k] = s.ok ? sm.table[ch][px[k * C + ch]] : 0.f;
+            float* dst = o + ch * plane + (int64_t)i * kStep * Wo;
+            if constexpr (VW == 4)
+                *reinterpret_cast<float4*>(dst) = make_float4(v[0], v[1], v[2], v[3]);
+            else
+                *dst = v[0];
+        }
+    }
+}
+
 }  // namespace
 
 extern "C" int uem_tile_gather(const float* soft_store, const int32_t* id_store, int64_t num_tiles, int c, int Hs, int Ws,
@@ -343,4 +427,36 @@ extern "C" int uem_label_gather_u8(const uint8_t* raw_store, int64_t num_tiles, 
     if (!down_out || fused) return 0;
     // bit 1 is already set from every label of the window; the down-scale's own check would report the same labels as bit 0
     return uem_downscale_label_i64(label_out, n, Ho, Wo, scale, n_classes, ignore_label, min_ratio, down_out, nullptr, stream);
+}
+
+extern "C" int uem_image_gather_u8(const uint8_t* store, int64_t num_tiles, int Hs, int Ws, int C, const float* table,
+                                   const int64_t* tiles, const int32_t* windows, int n, int Ho, int Wo, float* out, int32_t* status,
+                                   void* stream) {
+    UEM_REQUIRE((store || num_tiles == 0) && table && tiles && windows && out && status && n >= 0 && n <= 65535 && num_tiles >= 0 &&
+                    Hs > 0 && Ws > 0 && Ho > 0 && Wo > 0,
+                "uem_image_gather_u8: bad arguments");
+    UEM_REQUIRE(C >= 1 && C <= 4, "uem_image_gather_u8: C = %d channels outside [1,4]", C);
+    if (n == 0) return 0;
+    const dim3 grid(uem_div_up(Wo, TX), uem_div_up(Ho, TY), n);
+    UEM_REQUIRE(grid.y <= 65535, "uem_image_gather_u8: output height %d too large", Ho);
+    const cudaStream_t st = (cudaStream_t)stream;
+    const bool vec = Wo % 4 == 0 && uem_aligned16(out);
+#define UEM_IMAGE_GATHER(C_)                                                                                                     \
+    do {                                                                                                                         \
+        if (vec)                                                                                                                 \
+            image_gather_kernel<C_, 4><<<grid, kThreads, 0, st>>>(store, num_tiles, Hs, Ws, table, tiles, windows, Ho, Wo, out,  \
+                                                                  status);                                                       \
+        else                                                                                                                     \
+            image_gather_kernel<C_, 1><<<grid, kThreads, 0, st>>>(store, num_tiles, Hs, Ws, table, tiles, windows, Ho, Wo, out,  \
+                                                                  status);                                                       \
+    } while (0)
+    switch (C) {
+        case 1: UEM_IMAGE_GATHER(1); break;
+        case 2: UEM_IMAGE_GATHER(2); break;
+        case 3: UEM_IMAGE_GATHER(3); break;
+        default: UEM_IMAGE_GATHER(4); break;
+    }
+#undef UEM_IMAGE_GATHER
+    UEM_CHECK_LAUNCH();
+    return 0;
 }

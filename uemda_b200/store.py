@@ -11,14 +11,19 @@ Resident source set: the source label files' bytes kept in HBM.  The loader deco
 widens it to int64 (train_ssl_uem.py:205,216, train_align_uem.py:147,150) and the step down-scales it again for the
 prototypes (alignment.py:86-90,484-509).  ``LabelStore.batch`` produces ``label_s`` and its DownscaleLabel cells in one
 launch (uem_label_gather_u8) from the same ``(index, y0, x0, code)`` per sample.
+
+Resident image set: the decoded images' bytes kept in HBM.  The loader crops / flips / rotates each image with its labels
+(augmentation.py:150-157), normalises it to fp32 and the step copies the batch to the device.  ``ImageStore.batch`` cuts the
+normalised batch in one launch (uem_image_gather_u8) from the same ``(index, y0, x0, code)``, so the host only draws them.
 """
+import numpy as np
 import torch
 
 from . import _lib as L
 from . import config
 from .ops import f32
 
-__all__ = ["TileStore", "LabelStore"]
+__all__ = ["TileStore", "LabelStore", "ImageStore"]
 
 _I32_MIN, _I32_MAX = -2 ** 31, 2 ** 31 - 1
 
@@ -248,3 +253,79 @@ class LabelStore:
                 # F.one_hot in the reference (alignment.py:502) rejects these
                 raise RuntimeError("Class values must be non-negative and smaller than num_classes.")
         return label, down
+
+
+class ImageStore:
+    """``raw``: (T,H,W,C) uint8, the decoded images' bytes as image files hold them (channels interleaved, C in [1,4]: RGB,
+    IRRG, RGB+IR), one allocation, zero until ``put``.  ``table``: (C,256) fp32 on the device, the byte -> value map of each
+    channel (``normalize_table`` for albumentations' Normalize; ``torch.arange(256.) / 255`` per channel for ToTensor),
+    validated here.  ``batch`` cuts a batch with the windows and codes of ``TileStore.batch`` (``TileStore.d4_code``), so the
+    same indices and windows cut the same pixels out of a ``TileStore`` / ``LabelStore`` of the same tiles."""
+
+    def __init__(self, num_tiles, height, width, channels, table, device=None):
+        channels = int(channels)
+        if not 1 <= channels <= 4:
+            raise ValueError("ImageStore: %d channels outside [1, 4]" % channels)
+        table = torch.as_tensor(table)
+        if tuple(table.shape) != (channels, 256):
+            raise ValueError("ImageStore: table must map each of the 256 byte values of each of the %d channels, shape (%d, 256) "
+                             "(got %s)" % (channels, channels, tuple(table.shape)))
+        if not table.is_floating_point():
+            raise TypeError("ImageStore: table must hold floating-point values (got %s)" % table.dtype)
+        device = _cuda_device(device, "ImageStore")
+        self.shape = (int(num_tiles), int(height), int(width), channels)
+        self.raw = torch.zeros(self.shape, dtype=torch.uint8, device=device)
+        self.table = table.to(device=device, dtype=torch.float32).contiguous()
+        # bit 0: a sample of a batch() named a tile outside the store or a window outside the tile
+        self.status = torch.zeros(1, dtype=torch.int32, device=device)
+
+    @property
+    def device(self):
+        return self.raw.device
+
+    @staticmethod
+    def normalize_table(mean, std, max_pixel_value=255.0):
+        """(C,256) fp32 table of albumentations' ``Normalize(mean, std, max_pixel_value)`` with its arithmetic, in float32:
+        ``(v - mean * max_pixel_value) * reciprocal(std * max_pixel_value)``."""
+        m = np.asarray(mean, dtype=np.float32) * np.float32(max_pixel_value)
+        s = np.asarray(std, dtype=np.float32) * np.float32(max_pixel_value)
+        r = np.reciprocal(s, dtype=np.float32)
+        v = np.arange(256, dtype=np.float32)
+        return torch.from_numpy(np.ascontiguousarray((v[None, :] - m[:, None]) * r[:, None], dtype=np.float32))
+
+    def put(self, tiles, images):
+        """Writes images (b,H,W,C) uint8 at the tile indices ``tiles`` (a sequence or a tensor of b indices), from the host
+        (pinned: the copies are asynchronous) or the device, on the current stream."""
+        if images.dtype != torch.uint8:
+            raise TypeError("put: image bytes must be uint8 (got %s)" % images.dtype)
+        if images.dim() != 4 or tuple(images.shape[1:]) != self.shape[1:]:
+            raise ValueError("put: images of shape %s do not fit a store of %s (b,H,W,C)" % (tuple(images.shape), self.shape))
+        for t, i, j in _runs(_tile_list(tiles, images.shape[0], self.shape[0])):
+            self.raw[t:t + j - i].copy_(images[i:j], non_blocking=True)
+
+    def batch(self, tiles, windows, size, out=None):
+        """Cuts one batch: image[s, ch] = table[ch][store[tiles[s], ..., ch] at window (y0, x0) = windows[s][:2] under code
+        windows[s][2]], size = (Ho, Wo) or an int.  Returns (n,C,Ho,Wo) fp32, written into ``out`` when given.  tiles (n,)
+        int64 / windows (n,3) int32 device tensors and ``out`` make the call capturable in a CUDA graph (with
+        config.strict_asserts off).  An out-of-range sample gets zero planes and sets bit 0 of ``status``; under
+        config.strict_asserts the call reads the word back, clears it and raises IndexError."""
+        Ho, Wo = _size(size)
+        tiles, windows = _stage(tiles, windows, self.device)
+        n = tiles.numel()
+        if windows.shape[0] != n:
+            raise ValueError("batch: %d tile indices but %d windows" % (n, windows.shape[0]))
+        T, H, W, C = self.shape
+        if out is None:
+            out = torch.empty((n, C, Ho, Wo), dtype=torch.float32, device=self.device)
+        elif (not torch.is_tensor(out) or out.shape != (n, C, Ho, Wo) or out.dtype != torch.float32 or out.device != self.device
+              or not out.is_contiguous()):
+            raise ValueError("batch: out must be a contiguous (%d,%d,%d,%d) fp32 tensor on %s" % (n, C, Ho, Wo, self.device))
+        lib = L.bind(self.raw)
+        L.check(lib.uem_image_gather_u8(L.ptr(self.raw), T, H, W, C, L.ptr(self.table), L.ptr(tiles), L.ptr(windows), n, Ho, Wo,
+                                        L.ptr(out), L.ptr(self.status), L.stream_of(self.raw)))
+        if config.strict_asserts:
+            if int(self.status.item()):
+                self.status.zero_()
+                raise IndexError("ImageStore.batch: a sample names a tile outside [0, %d) or a window outside the %dx%d tile"
+                                 % (T, H, W))
+        return out
